@@ -9,8 +9,12 @@ A "step" = forward + BCEWithLogitsLoss + backward of one batch (+ gradient all-r
   python bench.py --impl reference [...]                          # reference CPU path (oracle port) on the host cores
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N    # one rank per GPU (weak scaling)
 
-Prints ONE JSON line on rank 0.  The timed loop is repeated `--repeats` times (each window = exactly K steps between
-barrier + synchronize); `value` is the MEDIAN window, all windows are listed in `windows_ms`.
+Prints ONE JSON line on rank 0.  A timed window is exactly K steps between barrier + synchronize; `--repeats R` times
+R windows (default 1) and reports the MEDIAN window, all windows are listed in `windows_ms`.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32): `loss`,
+`logits` and `grad.<parameter name>` for every parameter (rank 0's shard).  The inputs and the initial parameters are
+seeded, so two builds of the project run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -419,8 +423,12 @@ def run_ours(args):
     kw = wl.forward_kwargs()
 
     def build(use_graph, allreduce=None):
-        return GraphedTrainStep(model, devb[0][0], devb[0][1], forward_kwargs=kw,
+        step = GraphedTrainStep(model, devb[0][0], devb[0][1], forward_kwargs=kw,
                                 allreduce=(world > 1) if allreduce is None else allreduce, use_graph=use_graph)
+        # a replay refills the gradient tensors allocated while its graph was captured; building the next step points
+        # the parameters' .grad elsewhere, so each captured step keeps its own
+        step.grads = {n: p.grad for n, p in model.named_parameters()} if step.graph is not None else None
+        return step
     try:
         gs = build(not args.no_graph)
         graphed = not args.no_graph
@@ -471,6 +479,7 @@ def run_ours(args):
     copy_stream = torch.cuda.Stream()
     d2h_stream = torch.cuda.Stream()
     slots = [gs, build(graphed)]
+    last_run = {}
 
     def make_feed(batches, readback):
         staged_ev = [torch.cuda.Event() for _ in range(2)]
@@ -496,6 +505,7 @@ def run_ours(args):
             slot = i % 2
             main.wait_event(staged_ev[slot])
             loss = slots[slot].run()
+            last_run["step"] = slots[slot]
             free_ev[slot].record(main)
             enqueue_copy(i + 1)                                # overlaps with this step's compute
             if readback:
@@ -512,6 +522,8 @@ def run_ours(args):
     # ---- value: inputs resident in HBM when the timed region starts
     ms_dev, wins_dev = timed(make_feed(devb, False), args.steps, W, args.repeats)
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_run["step"], model)
     # ---- e2e: pinned host buffers -> H2D inside the timed region, loss read back every step
     ms_e2e, wins_e2e = timed(make_feed(host, True), args.steps, W, args.repeats)
     log(f"timing done: {ms_dev:.4f} ms/step device-resident, {ms_e2e:.4f} ms/step e2e")
@@ -655,6 +667,17 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, step, model):
+    """loss, logits and parameter gradients of the last run of `step` -> out_dir/<name>.npy (float32)"""
+    import numpy as np
+    grads = step.grads if step.grads is not None else {n: p.grad for n, p in model.named_parameters()}
+    arrays = {"loss": step.loss, "logits": step.logits}
+    arrays.update((f"grad.{n}", g) for n, g in grads.items() if g is not None)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 PROF_SLOTS = ("phi_pool_fwd_kernel", "phi_bwd_chain_kernel", "phi_wgrad_kernel", "gnn_conv_fwd_kernel",
               "gnn_conv_bwd_kernel", "gnn_agg_bwd_kernel", "knn_tiled_kernel", "gnn_fc1_bwd_kernel")
 KERNEL_SYMBOL = {"phi_pool_fwd_kernel": "phi_pool_fwd_pair_kernel"}   # H = 256 + max pooling runs the CTA-pair variant
@@ -741,7 +764,7 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=10)
-    ap.add_argument("--repeats", type=int, default=5, help="timed windows of --steps steps; the median is reported")
+    ap.add_argument("--repeats", type=int, default=1, help="timed windows of --steps steps; the median is reported")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="deepsets", choices=["deepsets", "yaml", "ragged", "graphnet", "sweep"])
     ap.add_argument("--batch", type=int, default=None, help="sets / graphs per GPU (default 256)")
@@ -749,7 +772,11 @@ def main():
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-baselines", action="store_true", help="skip the CPU / eager-GPU / wrapper-loop comparator legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, logits and gradients of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "sweep"):
+        ap.error("--dump-outputs needs --impl ours and a single-workload --config")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,6 @@
 // Shared definitions of the fused tcgen05 DeepSets kernels (forward, backward chain, wgrad).
 #pragma once
+#include "pcc_act_bf16.cuh"
 #include "pcc_common.cuh"
 #include "pcc_tc.cuh"
 
@@ -20,11 +21,6 @@ constexpr int kEpiThreads = kEpiWarps * 32;
 // [2][R][8] image.  A slab of a weight image is R = H rows x 128 B and is the unit streamed
 // through the smem ring; an activation tile is R = 128 rows.
 __host__ __device__ constexpr uint32_t w_slab_bytes(int H) { return (uint32_t)H * 128u; }
-constexpr uint32_t kActSlab = kTileM * 128u;  // 16 KB: 128 rows x 64 features
-// byte offset of the 16-byte chunk holding columns [col0, col0+8) of row r in a 128-row SW128 image
-__device__ __forceinline__ uint32_t act_chunk_off(int r, int col0) {
-  return (uint32_t)(col0 >> 6) * kActSlab + (uint32_t)r * 128u + ((uint32_t)(((col0 & 63) >> 3) ^ (r & 7)) << 4);
-}
 
 struct PhiParams {
   const float* x;
@@ -147,107 +143,11 @@ static __global__ void zero_u64_kernel(unsigned long long* p, int64_t n) {
 }
 
 // ------------------------------------------------------------------ helpers
-// Activation math of the bf16 path.  The epilogues are issue/MUFU bound (an exp/rcp based erf was measured
-// 1.5x SLOWER than erff(): two MUFU ops per element at quarter rate), so every activation costs ONE MUFU op:
-//   SiLU: sigmoid(z) = 0.5 (1 + tanh(z/2)) with tanh.approx (abs error ~5e-4);
-//   GELU: 0.5 z (1 + tanh(sqrt(2/pi) (z + 0.044715 z^3))) with tanh.approx — within 5e-4 (absolute) of the
-//         reference's exact-erf nn.GELU(), i.e. below the bf16 rounding (4e-3 relative) of the stored
-//         activation; the fp32 parity path (pcc_common.cuh) keeps the exact erf form;
-// and act / act' share the tanh where both are needed.
-__device__ __forceinline__ float tanh_approx(float x) {
-  float y;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-template <int ACT>
-__device__ __forceinline__ void act_and_grad_t(float z, float& a, float& da) {
-  if (ACT == PCC_ACT_RELU) {
-    a = fmaxf(z, 0.f);
-    da = z > 0.f ? 1.f : 0.f;
-  } else if (ACT == PCC_ACT_GELU) {
-    const float z2 = z * z;
-    const float t = tanh_approx(0.7978845608028654f * z * fmaf(0.044715f, z2, 1.f));
-    const float h = 0.5f * (1.f + t);
-    a = z * h;
-    da = h + 0.5f * z * (1.f - t * t) * (0.7978845608028654f * fmaf(0.134145f, z2, 1.f));
-  } else if (ACT == PCC_ACT_SILU) {
-    const float s = 0.5f * (1.f + tanh_approx(0.5f * z));
-    a = z * s;
-    da = s * (1.f + z * (1.f - s));
-  } else {
-    a = z;
-    da = 1.f;
-  }
-}
-template <int ACT>
-__device__ __forceinline__ float act_t(float z) {
-  if (ACT == PCC_ACT_RELU) return fmaxf(z, 0.f);
-  if (ACT == PCC_ACT_GELU) return 0.5f * z * (1.f + tanh_approx(0.7978845608028654f * z * fmaf(0.044715f, z * z, 1.f)));
-  if (ACT == PCC_ACT_SILU) return z * (0.5f * (1.f + tanh_approx(0.5f * z)));
-  return z;
-}
-
-// ---- packed-pair (f32x2) activation math.  The gelu / silu epilogues are bound by instruction issue (a trace of the
-// backward chain: 19k of 29k cycles per tile are activation math at ~20 scalar instructions per element); Blackwell's
-// packed fp32 pipe evaluates the polynomial parts of two elements per instruction, the tanh stays one MUFU op per element.
-__device__ __forceinline__ uint64_t fmul2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t fadd2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t splat2(float v) { return f32x2(v, v); }
-__device__ __forceinline__ uint64_t tanh2(uint64_t x) {
-  float lo, hi;
-  f32x2_unpack(x, lo, hi);
-  return f32x2(tanh_approx(lo), tanh_approx(hi));
-}
-// a = act(z), da = act'(z) for a pair; same functions of z as act_and_grad_t (identical operation order up to fma contraction)
-template <int ACT>
-__device__ __forceinline__ void act_and_grad2(uint64_t z, uint64_t& a, uint64_t& da) {
-  if (ACT == PCC_ACT_GELU) {
-    constexpr float c0 = 0.7978845608028654f;
-    const uint64_t z2 = fmul2(z, z);
-    const uint64_t t = tanh2(fmul2(z, ffma2(splat2(c0 * 0.044715f), z2, splat2(c0))));
-    const uint64_t h = ffma2(splat2(0.5f), t, splat2(0.5f));
-    a = fmul2(z, h);
-    // da = h + 2 z h (1 - h) u',  u' = c0 (1 + 0.134145 z^2)      (1 - t^2 = 4 h (1 - h))
-    const uint64_t up2 = ffma2(splat2(2.f * c0 * 0.134145f), z2, splat2(2.f * c0));
-    const uint64_t omh = ffma2(h, splat2(-1.f), splat2(1.f));
-    da = ffma2(fmul2(a, omh), up2, h);
-  } else if (ACT == PCC_ACT_SILU) {
-    const uint64_t s = ffma2(splat2(0.5f), tanh2(fmul2(z, splat2(0.5f))), splat2(0.5f));
-    a = fmul2(z, s);
-    da = ffma2(a, ffma2(s, splat2(-1.f), splat2(1.f)), s);   // s + z s (1 - s)
-  } else {
-    float lo, hi;
-    f32x2_unpack(z, lo, hi);
-    a = f32x2(fmaxf(lo, 0.f), fmaxf(hi, 0.f));
-    da = f32x2(lo > 0.f ? 1.f : 0.f, hi > 0.f ? 1.f : 0.f);
-  }
-}
-template <int ACT>
-__device__ __forceinline__ uint64_t act2(uint64_t z) {
-  if (ACT == PCC_ACT_GELU) {
-    constexpr float c0 = 0.7978845608028654f;
-    const uint64_t t = tanh2(fmul2(z, ffma2(splat2(c0 * 0.044715f), fmul2(z, z), splat2(c0))));
-    return fmul2(z, ffma2(splat2(0.5f), t, splat2(0.5f)));
-  }
-  if (ACT == PCC_ACT_SILU) return fmul2(z, ffma2(splat2(0.5f), tanh2(fmul2(z, splat2(0.5f))), splat2(0.5f)));
-  float lo, hi;
-  f32x2_unpack(z, lo, hi);
-  return f32x2(fmaxf(lo, 0.f), fmaxf(hi, 0.f));
-}
 __device__ __forceinline__ uint32_t pack_bf16x2_pair(uint64_t v) {
   float lo, hi;
   f32x2_unpack(v, lo, hi);
   return pack_bf16x2(lo, hi);
 }
-__device__ __forceinline__ uint64_t bf16x2_to_f32x2(uint32_t u) { return f32x2(bf16_lo(u), bf16_hi(u)); }
 
 __device__ __forceinline__ uint32_t float_ordered(float v) {
   uint32_t b = __float_as_uint(v);
@@ -256,14 +156,6 @@ __device__ __forceinline__ uint32_t float_ordered(float v) {
 __device__ __forceinline__ float ordered_float(uint32_t o) {
   uint32_t b = (o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o;
   return __uint_as_float(b);
-}
-
-
-template <int ACT>
-__device__ __forceinline__ float act_grad_t(float z) {
-  float a, da;
-  act_and_grad_t<ACT>(z, a, da);
-  return da;
 }
 
 int check_phi_desc(const pcc_phi_desc* d, const char* where);

@@ -350,8 +350,8 @@ __global__ void __launch_bounds__(kConvThreads, 1) gnn_conv_fwd_kernel(const Con
         // the A image is free once the MMAs of the previous tile have completed
         if (i == 0 && it >= 1) mbar_wait_b(empty, (uint32_t)((it - 1) & 1));
         const int col = 4 * lane;
-        *reinterpret_cast<uint2*>(Aimg + img_chunk_off(r, col) + ((col & 7) << 1)) = ag;
-        *reinterpret_cast<uint2*>(Aimg + img_chunk_off(r, kC + col) + ((col & 7) << 1)) = root;
+        *reinterpret_cast<uint2*>(Aimg + act_chunk_off(r, col) + ((col & 7) << 1)) = ag;
+        *reinterpret_cast<uint2*>(Aimg + act_chunk_off(r, kC + col) + ((col & 7) << 1)) = root;
       }
       fence_proxy_async();
       mbar_arrive_warp(full);
@@ -372,7 +372,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) gnn_conv_fwd_kernel(const Con
         for (int s = 0; s < 2 * kC / 64; ++s)
 #pragma unroll
           for (int ks = 0; ks < 4; ++ks)
-            umma_bf16(tmem + buf * kC, make_smem_desc_sw128_k(a_base + s * kSlab + ks * 32),
+            umma_bf16(tmem + buf * kC, make_smem_desc_sw128_k(a_base + s * kActSlab + ks * 32),
                       make_smem_desc_sw128_k(w_base + s * (kC * 128) + ks * 32), IDESC, (s | ks) != 0);
         umma_commit(empty);
         umma_commit(&acc_full[buf]);
@@ -481,7 +481,7 @@ __device__ __forceinline__ void load_h_tile(const __nv_bfloat16* __restrict__ h,
     const int r = c >> 4, kc = c & 15;
     const int64_t node = tile * kTile + r;
     const uint4 v = node < M ? __ldg(reinterpret_cast<const uint4*>(h + (size_t)node * kC) + kc) : make_uint4(0u, 0u, 0u, 0u);
-    *reinterpret_cast<uint4*>(img + img_chunk_off(r, kc * 8)) = v;
+    *reinterpret_cast<uint4*>(img + act_chunk_off(r, kc * 8)) = v;
   }
 }
 
@@ -538,7 +538,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) gnn_fc1_pool_fwd_kernel(const F
         for (int s = 0; s < kC / 64; ++s)
 #pragma unroll
           for (int ks = 0; ks < 4; ++ks)
-            umma_bf16(tmem + buf * kFc, make_smem_desc_sw128_k(h_base + buf * kHImg + s * kSlab + ks * 32),
+            umma_bf16(tmem + buf * kFc, make_smem_desc_sw128_k(h_base + buf * kHImg + s * kActSlab + ks * 32),
                       make_smem_desc_sw128_k(w_base + s * (kFc * 128) + ks * 32), IDESC, (s | ks) != 0);
         umma_commit(&empty[buf]);
         umma_commit(&acc_full[buf]);

@@ -14,6 +14,7 @@
 // and the mirrored backward (pcc_gnn_bwd.cu).  Activations between kernels: fp32 pre-activations z (needed by act'
 // and the BatchNorm backward), bf16 normalised activations h (the GEMM / gather operands).
 #pragma once
+#include "pcc_act_bf16.cuh"
 #include "pcc_common.cuh"
 #include "pcc_tc.cuh"
 
@@ -24,91 +25,6 @@ using namespace tc;
 constexpr int kC = 128;              // hidden width of the fused path
 constexpr int kFc = 256;             // fc1 width (hard-coded in the reference, graph_net.py:61)
 constexpr int kTile = 128;           // nodes per tile (= UMMA M)
-constexpr uint32_t kSlab = kTile * 128u;   // one 64-column slab of a 128-row SW128 image: 16 KB
-
-// Activation math of the bf16 path: ONE MUFU op per element (the kernels are issue bound, libm tanhf / erff cost ~30
-// instructions each and dominated the first version of every epilogue):
-//   tanh: tanh.approx.f32 (abs error ~5e-4, below the bf16 rounding of the stored activation);
-//   gelu: 0.5 z (1 + tanh(sqrt(2/pi) (z + 0.044715 z^3))) with tanh.approx — within 5e-4 of the reference's exact-erf
-//         nn.GELU() (graph_net.py:43); the fp32 mode of the module keeps libm (pcc_common.cuh).
-// Forward and backward use the same functions, so act' is consistent with the act the forward applied.
-__device__ __forceinline__ float tanh_fast(float x) {
-  float y;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-template <int ACT>
-__device__ __forceinline__ float actf(float z) {
-  if (ACT == PCC_ACT_RELU) return fmaxf(z, 0.f);
-  if (ACT == PCC_ACT_TANH) return tanh_fast(z);
-  if (ACT == PCC_ACT_GELU) return 0.5f * z * (1.f + tanh_fast(0.7978845608028654f * z * fmaf(0.044715f, z * z, 1.f)));
-  return z;
-}
-// act'(z), given a = act(z) where that is cheaper
-template <int ACT>
-__device__ __forceinline__ float actg(float z, float a) {
-  if (ACT == PCC_ACT_RELU) return z > 0.f ? 1.f : 0.f;
-  if (ACT == PCC_ACT_TANH) return 1.f - a * a;
-  if (ACT == PCC_ACT_GELU) {
-    const float z2 = z * z;
-    const float t = tanh_fast(0.7978845608028654f * z * fmaf(0.044715f, z2, 1.f));
-    return 0.5f * (1.f + t) + 0.5f * z * (1.f - t * t) * (0.7978845608028654f * fmaf(0.134145f, z2, 1.f));
-  }
-  return 1.f;
-}
-
-// ---- the same activations on packed pairs (f32x2): the polynomial parts of two elements per instruction, the tanh one
-// MUFU op per element.  Same formulas as actf / actg, so forward, backward and both code shapes agree.
-__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t spl2(float v) { return f32x2(v, v); }
-__device__ __forceinline__ uint64_t tanh2_fast(uint64_t x) {
-  float lo, hi;
-  f32x2_unpack(x, lo, hi);
-  return f32x2(tanh_fast(lo), tanh_fast(hi));
-}
-template <int ACT>
-__device__ __forceinline__ uint64_t actf2(uint64_t z) {
-  if (ACT == PCC_ACT_TANH) return tanh2_fast(z);
-  if (ACT == PCC_ACT_GELU) {
-    constexpr float c0 = 0.7978845608028654f;
-    const uint64_t t = tanh2_fast(mul2(z, ffma2(spl2(c0 * 0.044715f), mul2(z, z), spl2(c0))));
-    return mul2(z, ffma2(spl2(0.5f), t, spl2(0.5f)));
-  }
-  float lo, hi;
-  f32x2_unpack(z, lo, hi);
-  if (ACT == PCC_ACT_RELU) return f32x2(fmaxf(lo, 0.f), fmaxf(hi, 0.f));
-  return z;
-}
-// a = act(z), g = act'(z)
-template <int ACT>
-__device__ __forceinline__ void act_grad2(uint64_t z, uint64_t& a, uint64_t& g) {
-  if (ACT == PCC_ACT_TANH) {
-    a = tanh2_fast(z);
-    g = ffma2(mul2(a, spl2(-1.f)), a, spl2(1.f));
-  } else if (ACT == PCC_ACT_GELU) {
-    constexpr float c0 = 0.7978845608028654f;
-    const uint64_t z2 = mul2(z, z);
-    const uint64_t t = tanh2_fast(mul2(z, ffma2(spl2(c0 * 0.044715f), z2, spl2(c0))));
-    const uint64_t h = ffma2(spl2(0.5f), t, spl2(0.5f));                       // 0.5 (1 + t)
-    a = mul2(z, h);
-    // 0.5 z (1 - t^2) u' with u' = c0 (1 + 0.134145 z^2);  0.5 (1 - t^2) = 2 h (1 - h)
-    const uint64_t up2 = ffma2(spl2(2.f * c0 * 0.134145f), z2, spl2(2.f * c0));
-    const uint64_t omh = ffma2(h, spl2(-1.f), spl2(1.f));
-    g = ffma2(mul2(a, omh), up2, h);
-  } else if (ACT == PCC_ACT_RELU) {
-    float lo, hi;
-    f32x2_unpack(z, lo, hi);
-    a = f32x2(fmaxf(lo, 0.f), fmaxf(hi, 0.f));
-    g = f32x2(lo > 0.f ? 1.f : 0.f, hi > 0.f ? 1.f : 0.f);
-  } else {
-    a = z;
-    g = spl2(1.f);
-  }
-}
 
 // Sum over the 32 lanes of a warp of 32 per-lane values, transposed: afterwards v[0] of lane l holds the sum over
 // all lanes of their v[l] (31 shuffles instead of 160).
@@ -140,23 +56,12 @@ __device__ __forceinline__ float warp_transpose_sum16(float (&v)[16], int lane) 
   return v[0] + __shfl_xor_sync(0xffffffffu, v[0], 16);
 }
 
-// byte offset of the 16-byte chunk holding columns [col0, col0+8) of row r in a 128-row SW128 image
-__device__ __forceinline__ uint32_t img_chunk_off(int r, int col0) {
-  return (uint32_t)(col0 >> 6) * kSlab + (uint32_t)r * 128u + ((uint32_t)(((col0 & 63) >> 3) ^ (r & 7)) << 4);
-}
-
 __device__ __forceinline__ float2 bf2_to_f2(uint32_t u) { return make_float2(bf16_lo(u), bf16_hi(u)); }
 
 // ---- reduction of the landed rows of a gather slot (conv forward, aggregation backward): lane owns 4 channels = 8
 // bytes of every 256-byte row.  Both gather kernels are issue bound (ncu: 60-65 % issue-slot utilisation, half of the
 // samples in this loop), so the loop is written for instruction count: packed f32x2 adds (3 instructions per bf16
 // pair: two unpacks, one add), two independent chains, and no weight broadcast when the graph is unweighted.
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
-__device__ __forceinline__ uint64_t bf2_to_f32x2(uint32_t u) { return f32x2(__uint_as_float(u << 16), __uint_as_float(u & 0xFFFF0000u)); }
 template <int ROWB>
 __device__ __forceinline__ void slot_reduce(const uint8_t* slot, int cnt, int lane, bool weighted, float cw, float (&acc)[4]) {
   uint64_t a01 = f32x2(acc[0], acc[1]), a23 = f32x2(acc[2], acc[3]);
@@ -170,24 +75,24 @@ __device__ __forceinline__ void slot_reduce(const uint8_t* slot, int cnt, int la
       const uint2 v1 = *reinterpret_cast<const uint2*>(p + (u + 1) * ROWB);
       const uint2 v2 = *reinterpret_cast<const uint2*>(p + (u + 2) * ROWB);
       const uint2 v3 = *reinterpret_cast<const uint2*>(p + (u + 3) * ROWB);
-      a01 = add2(a01, bf2_to_f32x2(v0.x)); a23 = add2(a23, bf2_to_f32x2(v0.y));
-      b01 = add2(b01, bf2_to_f32x2(v1.x)); b23 = add2(b23, bf2_to_f32x2(v1.y));
-      a01 = add2(a01, bf2_to_f32x2(v2.x)); a23 = add2(a23, bf2_to_f32x2(v2.y));
-      b01 = add2(b01, bf2_to_f32x2(v3.x)); b23 = add2(b23, bf2_to_f32x2(v3.y));
+      a01 = fadd2(a01, bf16x2_to_f32x2(v0.x)); a23 = fadd2(a23, bf16x2_to_f32x2(v0.y));
+      b01 = fadd2(b01, bf16x2_to_f32x2(v1.x)); b23 = fadd2(b23, bf16x2_to_f32x2(v1.y));
+      a01 = fadd2(a01, bf16x2_to_f32x2(v2.x)); a23 = fadd2(a23, bf16x2_to_f32x2(v2.y));
+      b01 = fadd2(b01, bf16x2_to_f32x2(v3.x)); b23 = fadd2(b23, bf16x2_to_f32x2(v3.y));
     }
 #pragma unroll 1
     for (; u < cnt; ++u) {
       const uint2 v0 = *reinterpret_cast<const uint2*>(p + u * ROWB);
-      a01 = add2(a01, bf2_to_f32x2(v0.x)); a23 = add2(a23, bf2_to_f32x2(v0.y));
+      a01 = fadd2(a01, bf16x2_to_f32x2(v0.x)); a23 = fadd2(a23, bf16x2_to_f32x2(v0.y));
     }
-    a01 = add2(a01, b01); a23 = add2(a23, b23);
+    a01 = fadd2(a01, b01); a23 = fadd2(a23, b23);
   } else {
 #pragma unroll 2
     for (int u = 0; u < cnt; ++u) {
       const uint2 v = *reinterpret_cast<const uint2*>(p + u * ROWB);
       const float wu = __shfl_sync(0xffffffffu, cw, u);
       const uint64_t w2 = f32x2(wu, wu);
-      a01 = ffma2(w2, bf2_to_f32x2(v.x), a01); a23 = ffma2(w2, bf2_to_f32x2(v.y), a23);
+      a01 = ffma2(w2, bf16x2_to_f32x2(v.x), a01); a23 = ffma2(w2, bf16x2_to_f32x2(v.y), a23);
     }
   }
   f32x2_unpack(a01, acc[0], acc[1]);

@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
         const int r = c >> 4, kc = c & 15;
         const int64_t node = tile * kTile + r;
         const uint4 v = node < p.M ? __ldg(reinterpret_cast<const uint4*>(p.h_in + (size_t)node * kC) + kc) : make_uint4(0u, 0u, 0u, 0u);
-        *reinterpret_cast<uint4*>(Himg + buf * kHImgB + img_chunk_off(r, kc * 8)) = v;
+        *reinterpret_cast<uint4*>(Himg + buf * kHImgB + act_chunk_off(r, kc * 8)) = v;
       }
       fence_proxy_async();
       mbar_arrive_warp(&full[buf]);
@@ -182,7 +182,7 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
           for (int s = 0; s < kC / 64; ++s)
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)
-              umma_bf16(tmem + T_Z, make_smem_desc_sw128_k(h_base + buf * kHImgB + s * kSlab + ks * 32),
+              umma_bf16(tmem + T_Z, make_smem_desc_sw128_k(h_base + buf * kHImgB + s * kActSlab + ks * 32),
                         make_smem_desc_sw128_k(w_base + s * (kFc * 128) + half * (128 * 128) + ks * 32), IDESC_Z, (s | ks) != 0);
           umma_commit(z_full);
         }
@@ -192,15 +192,15 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
         // dh2[rows, in] = sum_out dZ[rows, out] W[out, in]
 #pragma unroll
         for (int ks = 0; ks < kFc / 16; ++ks)
-          umma_bf16(tmem + T_DH, make_smem_desc_sw128_k(d_base + (ks >> 2) * kSlab + (ks & 3) * 32),
+          umma_bf16(tmem + T_DH, make_smem_desc_sw128_k(d_base + (ks >> 2) * kActSlab + (ks & 3) * 32),
                     make_smem_desc_sw128_mn(w_base + ks * 2048, kFc * 128), IDESC_DH, ks != 0);
         // dW[out, in] += sum_rows dZ[rows, out] h2[rows, in]   (two halves of 128 output features)
 #pragma unroll
         for (int o = 0; o < 2; ++o)
 #pragma unroll
           for (int ks = 0; ks < kTile / 16; ++ks)
-            umma_bf16(tmem + T_DW + o * kC, make_smem_desc_sw128_mn(d_base + o * (2 * kSlab) + ks * 2048, kSlab),
-                      make_smem_desc_sw128_mn(h_base + buf * kHImgB + ks * 2048, kSlab), IDESC_DW, (it | ks) != 0);
+            umma_bf16(tmem + T_DW + o * kC, make_smem_desc_sw128_mn(d_base + o * (2 * kActSlab) + ks * 2048, kActSlab),
+                      make_smem_desc_sw128_mn(h_base + buf * kHImgB + ks * 2048, kActSlab), IDESC_DW, (it | ks) != 0);
         umma_commit(&empty[buf]);
         umma_commit(dh_full);
       }
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
 #pragma unroll
     for (int c = 0; c < 2; ++c) { st2[c][0] = st2[c][1] = 0.f; db3[0][c] = db3[1][c] = 0.f; }
     const int row = q * 32 + lane;
-    uint32_t* stage = reinterpret_cast<uint32_t*>(Dimg + cg * kSlab + q * 32 * 128);   // 4 KB: rows of this quarter, slab cg
+    uint32_t* stage = reinterpret_cast<uint32_t*>(Dimg + cg * kActSlab + q * 32 * 128);   // 4 KB: rows of this quarter, slab cg
     int it = 0;
     uint32_t use = 0;
     for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
@@ -244,17 +244,17 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
 #pragma unroll
           for (int j = 0; j < 16; j += 2) {
             const int col = col0 + j;
-            const uint64_t z = add2(f32x2(__uint_as_float(v[j]), __uint_as_float(v[j + 1])), *reinterpret_cast<const uint64_t*>(b3 + col));
+            const uint64_t z = fadd2(f32x2(__uint_as_float(v[j]), __uint_as_float(v[j + 1])), *reinterpret_cast<const uint64_t*>(b3 + col));
             uint64_t a, g;
-            act_grad2<ACT>(z, a, g);
+            act_and_grad2<ACT>(z, a, g);
             const uint64_t da = ffma2(*reinterpret_cast<const uint64_t*>(nK2 + col), a,
-                                      add2(f32x2(gq[c * 16 + j], gq[c * 16 + j + 1]), *reinterpret_cast<const uint64_t*>(nK1 + col)));
-            f32x2_unpack(mul2(da, g), dz[j], dz[j + 1]);
+                                      fadd2(f32x2(gq[c * 16 + j], gq[c * 16 + j + 1]), *reinterpret_cast<const uint64_t*>(nK1 + col)));
+            f32x2_unpack(fmul2(da, g), dz[j], dz[j + 1]);
             if (!valid) dz[j] = dz[j + 1] = 0.f;
           }
-          *reinterpret_cast<uint4*>(Dimg + img_chunk_off(row, col0)) =
+          *reinterpret_cast<uint4*>(Dimg + act_chunk_off(row, col0)) =
               make_uint4(pack_bf16x2(dz[0], dz[1]), pack_bf16x2(dz[2], dz[3]), pack_bf16x2(dz[4], dz[5]), pack_bf16x2(dz[6], dz[7]));
-          *reinterpret_cast<uint4*>(Dimg + img_chunk_off(row, col0 + 8)) =
+          *reinterpret_cast<uint4*>(Dimg + act_chunk_off(row, col0 + 8)) =
               make_uint4(pack_bf16x2(dz[8], dz[9]), pack_bf16x2(dz[10], dz[11]), pack_bf16x2(dz[12], dz[13]), pack_bf16x2(dz[14], dz[15]));
           db3[half][c] += warp_transpose_sum16(dz, lane);   // (bf16 rounding of dz not applied to the bias gradient)
         }
@@ -286,10 +286,10 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
 #pragma unroll
         for (int j = 0; j < 16; j += 2) {
           const uint64_t dh = valid ? f32x2(__uint_as_float(v[j]), __uint_as_float(v[j + 1])) : 0ull;
-          const uint64_t a = actf2<ACT>(f32x2(__uint_as_float(zp[c * 16 + j]), __uint_as_float(zp[c * 16 + j + 1])));
+          const uint64_t a = act2<ACT>(f32x2(__uint_as_float(zp[c * 16 + j]), __uint_as_float(zp[c * 16 + j + 1])));
           const uint64_t xh = ffma2(a, *reinterpret_cast<const uint64_t*>(r2 + col0 + j), *reinterpret_cast<const uint64_t*>(M2 + col0 + j));
           f32x2_unpack(dh, s1[j], s1[j + 1]);
-          f32x2_unpack(mul2(dh, xh), s2[j], s2[j + 1]);
+          f32x2_unpack(fmul2(dh, xh), s2[j], s2[j + 1]);
           out[c * 16 + j] = __float_as_uint(s1[j]);
           out[c * 16 + j + 1] = __float_as_uint(s1[j + 1]);
         }
@@ -497,10 +497,10 @@ __global__ void __launch_bounds__(kCbThreads, 1) gnn_conv_bwd_kernel(const ConvB
           a = actf<ACT>(z.w); dz[3] = sc.w * (g.w - c1.w - (a - mu.w) * rs.w * c2.w) * actg<ACT>(z.w, a);
         }
         db[0] += dz[0]; db[1] += dz[1]; db[2] += dz[2]; db[3] += dz[3];
-        *reinterpret_cast<uint2*>(Dimg + img_chunk_off(r, col) + ((col & 7) << 1)) =
+        *reinterpret_cast<uint2*>(Dimg + act_chunk_off(r, col) + ((col & 7) << 1)) =
             make_uint2(pack_bf16x2(dz[0], dz[1]), pack_bf16x2(dz[2], dz[3]));
-        *reinterpret_cast<uint2*>(Aimg + img_chunk_off(r, col) + ((col & 7) << 1)) = R.ag[j];
-        *reinterpret_cast<uint2*>(Aimg + img_chunk_off(r, kC + col) + ((col & 7) << 1)) = R.hr[j];
+        *reinterpret_cast<uint2*>(Aimg + act_chunk_off(r, col) + ((col & 7) << 1)) = R.ag[j];
+        *reinterpret_cast<uint2*>(Aimg + act_chunk_off(r, kC + col) + ((col & 7) << 1)) = R.hr[j];
       }
     };
     static_assert(kCbBatches == 4, "the pipeline below is written for 4 batches per tile");
@@ -549,12 +549,12 @@ __global__ void __launch_bounds__(kCbThreads, 1) gnn_conv_bwd_kernel(const ConvB
           tc_fence_after();
 #pragma unroll
           for (int ks = 0; ks < kC / 16; ++ks)
-            umma_bf16(tmem + T_DX, make_smem_desc_sw128_k(d_base + (ks >> 2) * kSlab + (ks & 3) * 32),
+            umma_bf16(tmem + T_DX, make_smem_desc_sw128_k(d_base + (ks >> 2) * kActSlab + (ks & 3) * 32),
                       make_smem_desc_sw128_mn(w_base + ks * 2048, kC * 128), IDESC_DX, ks != 0);
 #pragma unroll
           for (int ks = 0; ks < kTile / 16; ++ks)
-            umma_bf16(tmem + T_DW, make_smem_desc_sw128_mn(d_base + ks * 2048, kSlab),
-                      make_smem_desc_sw128_mn(a_base + ks * 2048, kSlab), IDESC_DW, (it | ks) != 0);
+            umma_bf16(tmem + T_DW, make_smem_desc_sw128_mn(d_base + ks * 2048, kActSlab),
+                      make_smem_desc_sw128_mn(a_base + ks * 2048, kActSlab), IDESC_DW, (it | ks) != 0);
           umma_commit(empty);
           umma_commit(dx_full);
         }

@@ -7,7 +7,6 @@
 // [E,C] message tensor is ever materialised.
 #include "pcc_common.cuh"
 #include "pcc_scan.cuh"
-#include <stdlib.h>
 
 namespace pcc {
 
@@ -352,90 +351,7 @@ static inline int threads_per_node(int64_t C, bool vec4) {
   return t;
 }
 
-// ------------------------------------------------------------------ kNN
-// One warp serves QW query points of (normally) one cloud.  Every lane evaluates one
-// candidate per step for all QW queries; each query's running top-k lives distributed
-// across the warp (lane i holds the i-th best (d2, id)), insertion by shuffle.
-__device__ __forceinline__ bool lex_less(float da, int ia, float db, int ib) {
-  return da < db || (da == db && ia < ib);
-}
-
-template <int QW>
-__global__ void __launch_bounds__(256) knn_kernel(const float* __restrict__ pos, int64_t pos_stride,
-                                                  const int64_t* __restrict__ offsets, int64_t n, int64_t B, int k,
-                                                  int64_t* __restrict__ nbr, float* __restrict__ d2o) {
-  const int lane = threadIdx.x & 31;
-  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  const int64_t q0 = warp * QW;
-  if (q0 >= n) return;
-  float qx[QW], qy[QW], qz[QW];
-  int64_t cs[QW], ce[QW];
-  float ld[QW];   // this lane's list entry per query
-  int li[QW];
-  int64_t lo_all = n, hi_all = 0;
-#pragma unroll
-  for (int q = 0; q < QW; ++q) {
-    const int64_t r = q0 + q;
-    ld[q] = INFINITY;
-    li[q] = 0x7fffffff;
-    cs[q] = 0; ce[q] = 0;
-    qx[q] = qy[q] = qz[q] = 0.f;
-    if (r < n) {
-      qx[q] = __ldg(pos + r * pos_stride);
-      qy[q] = __ldg(pos + r * pos_stride + 1);
-      qz[q] = __ldg(pos + r * pos_stride + 2);
-      int64_t lo = 0, hi = B;
-      while (lo < hi) {
-        int64_t mid = (lo + hi) >> 1;
-        if (offsets[mid + 1] <= r) lo = mid + 1; else hi = mid;
-      }
-      if (lo < B) { cs[q] = offsets[lo]; ce[q] = offsets[lo + 1]; }
-      lo_all = cs[q] < lo_all ? cs[q] : lo_all;
-      hi_all = ce[q] > hi_all ? ce[q] : hi_all;
-    }
-  }
-  for (int64_t j0 = lo_all; j0 < hi_all; j0 += 32) {
-    const int64_t j = j0 + lane;
-    float px = 0.f, py = 0.f, pz = 0.f;
-    if (j < hi_all) {
-      px = __ldg(pos + j * pos_stride);
-      py = __ldg(pos + j * pos_stride + 1);
-      pz = __ldg(pos + j * pos_stride + 2);
-    }
-#pragma unroll
-    for (int q = 0; q < QW; ++q) {
-      const float dx = px - qx[q], dy = py - qy[q], dz = pz - qz[q];
-      const float d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
-      const float thr_d = __shfl_sync(0xffffffffu, ld[q], k - 1);
-      const int thr_i = __shfl_sync(0xffffffffu, li[q], k - 1);
-      bool pass = (j >= cs[q]) && (j < ce[q]) && (j != q0 + q) && lex_less(d, (int)j, thr_d, thr_i);
-      unsigned ballot = __ballot_sync(0xffffffffu, pass);
-      while (ballot) {
-        const int L = __ffs(ballot) - 1;
-        ballot &= ballot - 1;
-        const float cd = __shfl_sync(0xffffffffu, d, L);
-        const int ci = __shfl_sync(0xffffffffu, (int)j, L);
-        const float ud = __shfl_up_sync(0xffffffffu, ld[q], 1);
-        const int ui = __shfl_up_sync(0xffffffffu, li[q], 1);
-        if (lex_less(cd, ci, ld[q], li[q])) {  // my entry is worse than the candidate: shift or insert
-          if (lane > 0 && lex_less(cd, ci, ud, ui)) { ld[q] = ud; li[q] = ui; }
-          else { ld[q] = cd; li[q] = ci; }
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int q = 0; q < QW; ++q) {
-    const int64_t r = q0 + q;
-    if (r < n && lane < k) {
-      const bool valid = li[q] != 0x7fffffff;
-      nbr[r * k + lane] = valid ? (int64_t)li[q] : -1;
-      d2o[r * k + lane] = valid ? ld[q] : INFINITY;
-    }
-  }
-}
-
-// ------------------------------------------------------------------ kNN, shared-memory tiled (the default)
+// ------------------------------------------------------------------ kNN, shared-memory tiled
 // CTA = 256 consecutive query points; for every cloud the CTA's queries belong to, the cloud's points stream through a
 // shared-memory tile ({x, y, z} as float4, 1024 candidates) that ALL warps read (one broadcast LDS.128 per candidate
 // instead of per-lane global loads).  Thread = one query: its running top-K lives in REGISTERS as a sorted list of
@@ -674,17 +590,8 @@ extern "C" int pcc_knn(const float* pos, int64_t pos_stride, const int64_t* offs
   PCC_REQUIRE(k >= 1 && k <= 32, "k must be in [1,32]");
   PCC_REQUIRE(n < (int64_t)0x7fffffff, "point count exceeds int32 range");
   if (n == 0) return 0;
-  static int legacy = -1;   // PCC_KNN_LEGACY=1: the warp-per-4-queries kernel of round 1 (kept for comparison)
-  if (legacy < 0) { const char* e = getenv("PCC_KNN_LEGACY"); legacy = (e && e[0] == '1') ? 1 : 0; }
   cudaStream_t st = (cudaStream_t)stream;
   ProfScope prof(6, st);
-  if (legacy) {
-    PCC_REQUIRE(nbr32 == nullptr, "the legacy kNN kernel has no int32 neighbour output");
-    constexpr int QW = 4;
-    const int64_t warps = cdiv(n, QW);
-    pcc::note_launch(1), knn_kernel<QW><<<(unsigned)cdiv(warps, 8), 256, 0, st>>>(pos, pos_stride, offsets, n, B, k, nbr, d2);
-    return check_launch(__func__);
-  }
   const unsigned grid = (unsigned)cdiv(n, 256);
   pcc::note_launch(1);
   // queue depth 16 (measured at N = 1024: depth 8 0.478 ms, 12 0.440 ms, 16 0.430 ms)

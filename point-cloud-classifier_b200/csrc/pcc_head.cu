@@ -13,6 +13,7 @@
 //                        g_{l-1} = dz_l W_l                            (tiles over [M,   K_l])
 // No atomics, no zero-fill launches, bitwise deterministic.
 #include "pcc_head.cuh"
+#include "pcc_tf32.cuh"
 
 namespace pcc {
 
@@ -20,30 +21,6 @@ constexpr int kHeadMaxDim = 1024;
 constexpr int kHeadMaxLayers = 4;
 constexpr int kHT = 32;    // output tile edge
 constexpr int kHThreads = 256;
-
-// hi = x truncated to TF32 (top 19 bits), lo = x - hi (exact in fp32; the tensor core reads its top 19 bits).
-// `cvt.rna.tf32.f32` is emulated with ~6 ALU instructions on this part — the rounding conversion made the split
-// 13 instructions per operand element and the kernels ALU bound (profiles/notes_r1.md); truncation costs 2 and
-// leaves a relative error of ~2^-20 per product.
-__device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
-  hi = __float_as_uint(x) & 0xffffe000u;
-  lo = __float_as_uint(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-// four consecutive floats p[0..3]; `nvalid` leading ones are in range; one 128-bit load when possible
-__device__ __forceinline__ float4 head_ld4(const float* p, bool vec, int nvalid) {
-  if (vec && nvalid == 4) return __ldg(reinterpret_cast<const float4*>(p));
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (nvalid > 0) v.x = __ldg(p);
-  if (nvalid > 1) v.y = __ldg(p + 1);
-  if (nvalid > 2) v.z = __ldg(p + 2);
-  if (nvalid > 3) v.w = __ldg(p + 3);
-  return v;
-}
 
 // One 32 x 32 output tile per CTA, K consumed in chunks of 256.  The kernel runs once per CTA with 8 warps on an
 // otherwise empty SM, so it is bound by dependent-latency chains, not by throughput (tools/head_micro.py: 3.2 us

@@ -215,6 +215,12 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_
 __host__ __device__ __forceinline__ uint32_t sw128_off(uint32_t row, uint32_t col, uint32_t R) {
   return (col >> 6) * (R * 128u) + row * 128u + ((((col & 63u) >> 3) ^ (row & 7u)) << 4) + ((col & 7u) << 1);
 }
+// Activation and gradient tiles are 128-row images: one 64-column slab is 16 KB.
+constexpr uint32_t kActSlab = 128u * 128u;
+// byte offset of the 16-byte chunk holding columns [col0, col0+8) of row r in a 128-row SW128 image
+__device__ __forceinline__ uint32_t act_chunk_off(int r, int col0) {
+  return (uint32_t)(col0 >> 6) * kActSlab + (uint32_t)r * 128u + ((uint32_t)(((col0 & 63) >> 3) ^ (r & 7)) << 4);
+}
 // K-major view [R x K]: start = slab base + 32 B per UMMA K step inside the slab; SBO = 1024 (8-row groups)
 __device__ __forceinline__ uint64_t make_smem_desc_sw128_k(uint32_t saddr) {
   uint64_t d = 0;
@@ -282,8 +288,20 @@ __device__ __forceinline__ uint64_t ffma2(uint64_t a, uint64_t b, uint64_t c) {
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
   return d;
 }
+__device__ __forceinline__ uint64_t fmul2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
+__device__ __forceinline__ uint64_t fadd2(uint64_t a, uint64_t b) {
+  uint64_t d;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
+__device__ __forceinline__ uint64_t splat2(float v) { return f32x2(v, v); }
 __device__ __forceinline__ float bf16_lo(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t u) { return __uint_as_float(u & 0xFFFF0000u); }
+__device__ __forceinline__ uint64_t bf16x2_to_f32x2(uint32_t u) { return f32x2(bf16_lo(u), bf16_hi(u)); }
 
 }  // namespace tc
 }  // namespace pcc

@@ -82,8 +82,9 @@ def graphconv(sd, prefix: str, x, edges, weights, aggr: str, q=None) -> torch.Te
     return F.linear(agg, w_rel, sd[prefix + ".lin_rel.bias"]) + F.linear(x, w_root)
 
 
-def global_mean_pool(x: torch.Tensor, membership: torch.Tensor) -> torch.Tensor:
-    B = int(membership.max()) + 1
+def global_mean_pool(x: torch.Tensor, membership: torch.Tensor, num_graphs: Optional[int] = None) -> torch.Tensor:
+    """num_graphs (PyG's `size`): defaults to membership.max() + 1; a graph without nodes pools to 0"""
+    B = int(membership.max()) + 1 if num_graphs is None else int(num_graphs)
     out = x.new_zeros((B, x.shape[1])).index_add(0, membership, x)
     cnt = torch.zeros(B, dtype=x.dtype, device=x.device).index_add(0, membership, torch.ones_like(membership, dtype=x.dtype))
     return out / cnt.clamp(min=1.0).view(-1, 1)
@@ -107,13 +108,14 @@ def _bn(sd, prefix: str, x: torch.Tensor, training: bool, stats_out: Optional[di
 
 def graphnet_forward(sd: Dict[str, torch.Tensor], cfg: dict, x, membership, edges, weights=None,
                      training: bool = True, stats_out: Optional[dict] = None,
-                     operand_rounding: Optional[str] = None) -> torch.Tensor:
+                     operand_rounding: Optional[str] = None, num_graphs: Optional[int] = None) -> torch.Tensor:
     """cfg keys = the reference ctor kwargs (graph_net.py:10-22); only the
     use_gat=False, sag_pool=False branch (configs/graph_net.yaml:6,8) is restated.
     operand_rounding="bf16": the STATED arithmetic of the product's bf16 GraphNet mode — the normalised activations h1
     (and h2 when fc1 runs per node, deepchem_style), the conv2 aggregate and the conv2 (/ fc1) weights are rounded to
     bf16; products and sums, pre-activations, BatchNorm statistics, conv1, the pooled tensors and the graph-level layers
-    stay fp32.  Same algorithm, stated operand precision."""
+    stay fp32.  Same algorithm, stated operand precision.
+    num_graphs: number of graphs of the batch (default membership.max() + 1; larger values append empty graphs)."""
     if cfg.get("use_gat", False) or cfg.get("sag_pool", False):
         raise NotImplementedError("GATConv / SAGPooling branches are out of scope (SURVEY.md §2 row 3)")
     act = cfg["activation"]
@@ -130,9 +132,9 @@ def graphnet_forward(sd: Dict[str, torch.Tensor], cfg: dict, x, membership, edge
     if cfg.get("deepchem_style", False):
         h = F.linear(h, q(sd["fc1.weight"]) if q is not None else sd["fc1.weight"], sd["fc1.bias"])
         h = _bn(sd, "bn3", _act(act, h), training, stats_out)
-        h = global_mean_pool(h, membership)
+        h = global_mean_pool(h, membership, num_graphs)
     else:
-        h = global_mean_pool(h, membership)
+        h = global_mean_pool(h, membership, num_graphs)
         h = F.linear(h, sd["fc1.weight"], sd["fc1.bias"])
         h = _bn(sd, "bn3", _act(act, h), training, stats_out)
     return F.linear(h, sd["fc2.weight"], sd["fc2.bias"])
@@ -144,11 +146,12 @@ TRAINABLE = ("conv1.lin_rel.weight", "conv1.lin_rel.bias", "conv1.lin_root.weigh
              "fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias")
 
 
-def graphnet_train_step(sd, cfg, x, membership, edges, weights, y, operand_rounding: Optional[str] = None):
+def graphnet_train_step(sd, cfg, x, membership, edges, weights, y, operand_rounding: Optional[str] = None,
+                        num_graphs: Optional[int] = None):
     leaves = {k: (v.detach().clone().requires_grad_(True) if k in TRAINABLE else v) for k, v in sd.items()}
     stats = {}
     logits = graphnet_forward(leaves, cfg, x, membership, edges, weights, training=True, stats_out=stats,
-                              operand_rounding=operand_rounding)
+                              operand_rounding=operand_rounding, num_graphs=num_graphs)
     loss = F.binary_cross_entropy_with_logits(logits, y)
     loss.backward()
     grads = {k: leaves[k].grad for k in TRAINABLE}

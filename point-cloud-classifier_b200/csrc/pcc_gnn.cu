@@ -179,7 +179,8 @@ __global__ void gnn_bn_eval_kernel(const float* __restrict__ running_mean, const
 }
 
 // per-graph mean + BatchNorm affine of the pooled sums: P = psum / max(n_g, 1), y = P * scale + shift   ([B, Cn] tensors;
-// global_mean_pool commutes with the affine, graph_net.py:89-92 / :96)
+// global_mean_pool commutes with the affine, graph_net.py:89-92 / :96).  A graph without nodes pools to y = 0, as
+// global_mean_pool of the normalised rows does: the affine is applied per node, so an empty graph never receives the shift.
 __global__ void gnn_pool_affine_kernel(const float* __restrict__ psum, const int64_t* __restrict__ counts,
                                        const float* __restrict__ scale, const float* __restrict__ shift, int64_t B, int Cn,
                                        float* __restrict__ P, float* __restrict__ y) {
@@ -190,7 +191,7 @@ __global__ void gnn_pool_affine_kernel(const float* __restrict__ psum, const int
   const int64_t n = counts[b];
   const float pv = psum[i] / (float)(n > 0 ? n : 1);
   P[i] = pv;
-  y[i] = fmaf(pv, scale[c], shift[c]);
+  y[i] = n > 0 ? fmaf(pv, scale[c], shift[c]) : 0.f;
 }
 
 // h = bf16( act(z) * scale + shift ), 8 elements per thread

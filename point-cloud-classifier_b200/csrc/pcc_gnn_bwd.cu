@@ -355,7 +355,8 @@ __global__ void __launch_bounds__(kFbThreads, 1) gnn_fc1_bwd_kernel(const Fc1Bwd
 //   sumG[c] = sum_b G, sumGx[c] = sum_b G xhat(P)      -> dbeta = sumG, dgamma = sumGx,
 //   gs[b, c] = G * f / n_b,  kap[c] = f * sumG / M,  lam[c] = f * sumGx / M      (f = s[c], or 1 when use_scale = 0)
 // are everything the node-level backward kernels need (da = gs[graph] - kap - lam xhat).  One CTA per 32 columns (32 row
-// slices per column, reduced through shared memory in a fixed order).
+// slices per column, reduced through shared memory in a fixed order).  An empty graph's y is the constant 0 (no node feeds
+// it): gs = 0 and it adds nothing to sumG / sumGx.
 __global__ void __launch_bounds__(1024) gnn_pool_bwd_prep_kernel(const float* __restrict__ G, const float* __restrict__ P,
                                                                 const float* __restrict__ mu, const float* __restrict__ rinv,
                                                                 const float* __restrict__ s, const int64_t* __restrict__ counts,
@@ -369,8 +370,10 @@ __global__ void __launch_bounds__(1024) gnn_pool_bwd_prep_kernel(const float* __
   if (c < Cn) {
     const float f = use_scale ? s[c] : 1.f, m = mu[c], r = rinv[c];
     for (int64_t b = sl; b < B; b += 32) {
-      const float g = G[b * Cn + c];
+      // the loads of n, G and P issue together (a select, no branch on n): the kernel is latency-bound
       const int64_t n = counts[b];
+      const float graw = G[b * Cn + c];
+      const float g = n > 0 ? graw : 0.f;
       gs[b * Cn + c] = g * f / (float)(n > 0 ? n : 1);
       a0 += g;
       a1 += g * ((P[b * Cn + c] - m) * r);

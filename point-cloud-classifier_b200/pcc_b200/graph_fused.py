@@ -40,6 +40,7 @@ class FusedGraph:
             raise ValueError("the fused GraphNet kernels index nodes and edges with int32")
         self.k_uniform = k_uniform
         self.block_offsets = block_offsets           # [B+1] node range per cloud of a block-diagonal simple graph, or None
+        weights = L.f32c(weights) if weights is not None else None    # the kernels read fp32 weights
         csr = None
         if by_dst is not None:                       # e.g. a kNN graph: k consecutive edges per target, already grouped
             self.rowptr_d, self.col_d = by_dst
@@ -117,6 +118,7 @@ class GraphNetFusedFn(torch.autograd.Function):
             (w_rel1, b_rel1, w_root1, w_rel2, b_rel2, w_root2, g1, be1, g2, be2) = params
             w_fc1 = b_fc1 = g3 = be3 = None
         x = L.f32c(x)
+        membership = L.i64c(membership)              # the kernels read int64 graph ids
         dev = L.require_cuda(x, membership, *params)
         st = L.stream_ptr(dev)
         M, F = x.shape

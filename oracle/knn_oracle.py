@@ -26,8 +26,23 @@ from __future__ import annotations
 import numpy as np
 
 
-def knn_neighbours(pos: np.ndarray, offsets: np.ndarray, k: int):
-    """pos[n,3] float32, offsets[B+1] int64 -> (nbr[n,k] int64 (-1 pad), d2[n,k] float32 (inf pad))."""
+def _sq_dist(q: np.ndarray, p: np.ndarray) -> np.ndarray:
+    """d2[i, j] = ((dx*dx + dy*dy) + dz*dz) between rows q[i] and p[j], every product and sum rounded to float32"""
+    dx = q[:, None, 0] - p[None, :, 0]
+    dy = q[:, None, 1] - p[None, :, 1]
+    dz = q[:, None, 2] - p[None, :, 2]
+    d2 = (dx * dx + dy * dy).astype(np.float32) + (dz * dz).astype(np.float32)
+    return d2.astype(np.float32)
+
+
+def knn_neighbours(pos: np.ndarray, offsets: np.ndarray, k: int, rows_per_chunk: int = None):
+    """pos[n,3] float32, offsets[B+1] int64 -> (nbr[n,k] int64 (-1 pad), d2[n,k] float32 (inf pad)).
+
+    rows_per_chunk: evaluate the centres of a cloud that many at a time, so memory stays at rows_per_chunk x cloud
+    size instead of cloud size squared (clouds of 16384 points).  Same float32 distances and the same selection,
+    so the result is identical: the k-th smallest distance of a row is found with a partition, every candidate at or
+    below it is kept in ascending id order (all ties at the boundary included) and a stable sort by distance of those
+    candidates keeps the first k."""
     pos = np.ascontiguousarray(pos, dtype=np.float32)
     n = pos.shape[0]
     nbr = np.full((n, k), -1, dtype=np.int64)
@@ -36,20 +51,33 @@ def knn_neighbours(pos: np.ndarray, offsets: np.ndarray, k: int):
         s, e = int(offsets[b]), int(offsets[b + 1])
         p = pos[s:e]
         m = e - s
+        kk = min(k, m - 1)
         if m == 0:
             continue
-        dx = p[:, None, 0] - p[None, :, 0]
-        dy = p[:, None, 1] - p[None, :, 1]
-        dz = p[:, None, 2] - p[None, :, 2]
-        d2 = (dx * dx + dy * dy).astype(np.float32) + (dz * dz).astype(np.float32)
-        d2 = d2.astype(np.float32)
-        np.fill_diagonal(d2, np.inf)
-        order = np.argsort(d2, axis=1, kind="stable")
-        kk = min(k, m - 1)
-        if kk > 0:
-            sel = order[:, :kk]
-            nbr[s:e, :kk] = sel + s
-            d2o[s:e, :kk] = np.take_along_axis(d2, sel, axis=1)
+        if rows_per_chunk is None:
+            d2 = _sq_dist(p, p)
+            np.fill_diagonal(d2, np.inf)
+            order = np.argsort(d2, axis=1, kind="stable")
+            if kk > 0:
+                sel = order[:, :kk]
+                nbr[s:e, :kk] = sel + s
+                d2o[s:e, :kk] = np.take_along_axis(d2, sel, axis=1)
+            continue
+        if kk <= 0:
+            continue
+        for r0 in range(0, m, rows_per_chunk):
+            r1 = min(r0 + rows_per_chunk, m)
+            d2 = _sq_dist(p[r0:r1], p)
+            rows = np.arange(r1 - r0)
+            d2[rows, rows + r0] = np.inf
+            kth = np.partition(d2, kk - 1, axis=1)[:, kk - 1:kk]
+            row, col = np.nonzero(d2 <= kth)                 # row-major: ids ascend inside every row
+            val = d2[row, col]
+            order = np.lexsort((col, val, row))             # by row, then distance, then id
+            first = np.concatenate([[0], np.cumsum(np.bincount(row, minlength=r1 - r0))[:-1]])
+            pick = order[(first[:, None] + np.arange(kk)[None, :]).reshape(-1)].reshape(r1 - r0, kk)
+            nbr[s + r0:s + r1, :kk] = col[pick] + s
+            d2o[s + r0:s + r1, :kk] = val[pick]
     return nbr, d2o
 
 

@@ -40,6 +40,7 @@ BF16_GRAD_TOL = 1e-2
 FP32_TOL = 1.5e-2
 FP32_GRAD_TOL_SMOOTH = 1e-2
 FP32_GRAD_TOL_RELU = 0.16
+LOSS_TOL = 2e-3   # |loss - loss of the bf16-operand oracle| <= LOSS_TOL * |that loss|, GraphedTrainStep's fused BCE
 
 
 def check_step_against_oracles(tag, act, named_grads, logits, ref32, ref16):

@@ -49,35 +49,23 @@ def _cfg(act, aggr, F=4, hidden=128, deepchem=True):
                 pool_ratio=0.5, local_pooling=aggr, global_pooling="mean", deepchem_style=deepchem)
 
 
-def _check_fused_step(cfg, x, memb, edges, w, y, *, num_graphs=None, fwd_kwargs={}, module=None):
-    """One bf16 train step (forward + BCE + backward) against the oracle with the stated bf16 operand rounding and the
-    fp32 oracle, the running statistics it leaves, and the eval-mode forward on those statistics.  module: a KnnGraphNet
-    (called as module(x, memb); `edges` is then the oracle's copy of the kNN graph it builds), else a GraphNet is built
-    from cfg and called on (x, memb, edges[, w]).  Returns the module and the train / eval logits."""
+def check_fused_step_against_oracles(cfg, sd, x, memb, edges, w, y, logits, grads, module, args, *, num_graphs=None,
+                                     fwd_kwargs={}):
+    """Compares one bf16 train step (forward + BCE + backward) that `module` ran from the parameters `sd` with the
+    oracle with the stated bf16 operand rounding and with the fp32 oracle, both on the host tensors (x, memb, edges, w,
+    y); then the running statistics the step left, and the eval-mode forward module(*args, num_graphs, **fwd_kwargs)
+    on those statistics.  logits: the train-mode logits; grads: {GraphNet parameter name: gradient}; module: the
+    GraphNet, or a KnnGraphNet (its GraphNet is module.net; `edges` is then the oracle's copy of the kNN graph it
+    builds).  Prints the errors, asserts the stated tolerances and returns the eval-mode logits."""
     act = cfg["activation"]
-    sd = GO.init_state_dict(cfg, seed=23)
+    net = getattr(module, "net", module)
     ref_logits, _, ref_grads, ref_stats = GO.graphnet_train_step(sd, cfg, x, memb, edges, w, y, num_graphs=num_graphs)
     q_logits, _, q_grads, _ = GO.graphnet_train_step(sd, cfg, x, memb, edges, w, y, operand_rounding="bf16",
                                                      num_graphs=num_graphs)
-
-    if module is None:
-        m = pcc_b200.GraphNet(**cfg, precision="bf16").cuda()
-        args = [x.cuda(), memb.cuda(), edges.cuda()] + ([w.cuda()] if w is not None else [])
-        net = m
-    else:
-        m = module.cuda()
-        args = [x.cuda(), memb.cuda()]
-        net = m.net
-    net.load_state_dict(sd)
-    m.train()
-    logits = m(*args, num_graphs=num_graphs, **fwd_kwargs)
-    assert net.last_path == "fused-bf16"
-    torch.nn.BCEWithLogitsLoss()(logits, y.cuda()).backward()
     e_log, e_logq = rel_err(logits, ref_logits), rel_err(logits, q_logits)
     worst, worstq, rows = ("", 0.0), ("", 0.0), []
-    params = dict(net.named_parameters())
     for kname, ref in ref_grads.items():
-        got = params[kname].grad
+        got = grads[kname]
         assert got is not None, kname
         e, eq = rel_l2(got, ref), rel_l2(got, q_grads[kname])
         rows.append(f"{kname}={eq:.1e}/{e:.1e}")
@@ -96,12 +84,39 @@ def _check_fused_step(cfg, x, memb, edges, w, y, *, num_graphs=None, fwd_kwargs=
     for kname, v in ref_stats.items():
         torch.testing.assert_close(new_sd[kname].cpu(), v, rtol=2e-2, atol=2e-3)
     # eval mode: running statistics
-    m.eval()
+    module.eval()
     with torch.no_grad():
-        ev = m(*args, num_graphs=num_graphs, **fwd_kwargs)
+        ev = module(*args, num_graphs=num_graphs, **fwd_kwargs)
     sd_eval = {kk: v.cpu() for kk, v in new_sd.items()}
     ref_ev = GO.graphnet_forward(sd_eval, cfg, x, memb, edges, w, training=False, num_graphs=num_graphs)
-    assert rel_err(ev, ref_ev) < LOGIT_TOL
+    e_ev = rel_err(ev, ref_ev)
+    print(f"  eval logits {e_ev:.1e} vs fp32 oracle on the running statistics; running statistics max |diff| "
+          f"{max(float((new_sd[kname].cpu().double() - v.double()).abs().max()) for kname, v in ref_stats.items()):.1e}")
+    assert e_ev < LOGIT_TOL
+    return ev
+
+
+def _check_fused_step(cfg, x, memb, edges, w, y, *, num_graphs=None, fwd_kwargs={}, module=None):
+    """One bf16 train step (forward + BCE + backward) through check_fused_step_against_oracles.  module: a KnnGraphNet
+    (called as module(x, memb); `edges` is then the oracle's copy of the kNN graph it builds), else a GraphNet is built
+    from cfg and called on (x, memb, edges[, w]).  Returns the module and the train / eval logits."""
+    sd = GO.init_state_dict(cfg, seed=23)
+    if module is None:
+        m = pcc_b200.GraphNet(**cfg, precision="bf16").cuda()
+        args = [x.cuda(), memb.cuda(), edges.cuda()] + ([w.cuda()] if w is not None else [])
+        net = m
+    else:
+        m = module.cuda()
+        args = [x.cuda(), memb.cuda()]
+        net = m.net
+    net.load_state_dict(sd)
+    m.train()
+    logits = m(*args, num_graphs=num_graphs, **fwd_kwargs)
+    assert net.last_path == "fused-bf16"
+    torch.nn.BCEWithLogitsLoss()(logits, y.cuda()).backward()
+    grads = {k: p.grad for k, p in net.named_parameters()}
+    ev = check_fused_step_against_oracles(cfg, sd, x, memb, edges, w, y, logits, grads, m, args, num_graphs=num_graphs,
+                                          fwd_kwargs=fwd_kwargs)
     return m, logits.detach(), ev
 
 
@@ -387,6 +402,8 @@ def test_knn_graphnet_module_uses_fused_path_and_matches_fp32_mode():
     ([1024] * 5, 20),
     ([33, 1300, 21, 2900], 20),          # clouds beyond one bitmap pass (> ~1250 points)
     ([64], 5),
+    ([16384, 300], 20),                  # the sweep's largest cloud: 245 bitmap passes
+    ([8192, 8192], 20),
 ])
 def test_csr_transpose_blocks_matches_numpy(sizes, k):
     """pcc_csr_transpose_blocks (per-cloud shared-memory transpose of a kNN graph) is bit-exact against a stable numpy
@@ -394,7 +411,7 @@ def test_csr_transpose_blocks_matches_numpy(sizes, k):
     import ctypes as C
     from pcc_b200 import _lib as L
     feats, memb, off = _clouds(sizes, seed=5)
-    nbr, _ = KO.knn_neighbours(feats[:, 1:4].numpy(), off, k)
+    nbr, _ = KO.knn_neighbours(feats[:, 1:4].numpy(), off, k, rows_per_chunk=1024)
     n = feats.shape[0]
     src = nbr.reshape(-1).astype(np.int64)                 # slot p = (target p // k) <- source nbr
     tgt = np.repeat(np.arange(n, dtype=np.int64), k)

@@ -126,6 +126,11 @@ int pcc_csr_transpose(const int32_t* col_d, const int64_t* rowptr_d, int64_t E, 
  * trap): one CTA per cloud in shared memory, no workspace, no sort. */
 int pcc_csr_transpose_blocks(const int32_t* col_d, int k, const int64_t* offsets, int64_t B, int64_t n, int64_t* rowptr_s,
                              int32_t* col_s, int device, void* stream);
+/* for such a transpose (k slots per target, no repeated edge, rows of col_s ascending): pos_s[E = n k] = the by-target slot
+ * of every by-source entry, pos_s[q] = t k + s where col_s[q] = t and col_d[t k + s] is the row's source (a missing entry
+ * traps).  Feeds pcc_gnn_agg_bwd with max aggregation. */
+int pcc_csr_transpose_pos(const int32_t* col_d, int k, int64_t n, const int64_t* rowptr_s, const int32_t* col_s, int32_t* pos_s,
+                          int device, void* stream);
 /* out[i,:] = aggr_{e in in(i)} w_e * x[src(e),:]   (aggr: PCC_POOL_ADD / MEAN / MAX);
  * rowptr/perm = CSR by TARGET.  arg_edge[n,C] (int32 edge id, -1 if none) for MAX only. */
 int pcc_graph_aggregate_fwd(const float* x, const int64_t* src, const float* w, const int64_t* rowptr,
@@ -225,15 +230,16 @@ int pcc_mlp_head_bwd(const pcc_head_desc* d, const float* x, const float* zsave,
                      float* const* dw, float* const* db, void* ws, int64_t M, int device, void* stream);
 
 /* ---- fused bf16 GraphNet path (tcgen05 / TMEM): the neighbour stage of /root/reference/models/graph_net.py:73-92 for
- *      hidden_dim = 128 (configs/graph_net.yaml), deepchem_style = true, aggregation add / mean, activations tanh / relu /
- *      gelu.  Pipeline and data layout: DESIGN.md section 4 (GraphNet) and csrc/pcc_gnn.cuh.  CSR arguments: rowptr[M+1]
+ *      hidden_dim = 128 (configs/graph_net.yaml), deepchem_style = true, aggregation add / mean / max (`aggr` =
+ *      PCC_POOL_ADD / MEAN / MAX), activations tanh / relu / gelu.  Pipeline and data layout: DESIGN.md section 4 (GraphNet) and csrc/pcc_gnn.cuh.  CSR arguments: rowptr[M+1]
  *      int64, col[E] int32 = neighbour node per CSR slot, w[E] fp32 edge weight per slot or NULL.  *_bf16 = bf16 [M,128]
  *      row-major.  "partials" are per-CTA partial sums, [nblk][...]; *nblk_out (host int) receives the block count used.
  *      Every buffer is caller-owned.
  *   pcc_gnn_pack_weights : conv2 lin_rel / lin_root [128,128] and fc1 [256,128] fp32 -> packed bf16 operand images
  *                          (pcc_gnn_packed_bytes() bytes); w_fc1 may be NULL.
  *   pcc_gnn_conv1_fwd    : GraphConv 1 (graph_net.py:73; K = 2 input_dim <= 16, CUDA cores): agg_out[M,F], z_out[M,128],
- *                          partials [nblk][2][128] = sums of act(z), act(z)^2 (BatchNorm statistics, :76).
+ *                          partials [nblk][2][128] = sums of act(z), act(z)^2 (BatchNorm statistics, :76).  MAX: agg = max
+ *                          of the fp32 products w_e x[src(e)], 0 for a node without in-edges.
  *   pcc_gnn_bn_finalize  : partial sums -> scale = gamma*invstd, shift = beta - mean*scale, mean, invstd; updates the
  *                          running statistics (momentum, unbiased variance) when the pointers are non-NULL.
  *   pcc_gnn_bn_eval      : scale / shift from the running statistics (eval mode).
@@ -243,12 +249,17 @@ int pcc_mlp_head_bwd(const pcc_head_desc* d, const float* x, const float* zsave,
  *                          sums in the epilogue; agg_out keeps the aggregate for the weight gradient.  Optional
  *                          membership + psum[B,128]: per-graph sums of act(z) (deepchem_style = false pools right after
  *                          the block, graph_net.py:96: mean pooling commutes with the BatchNorm affine).
+ *                          MAX: agg[i][c] = max over the row of i of the fp32 products w_e h[src(e)][c] (0 without in-edges),
+ *                          then rounded to bf16.  Ties: the FIRST position of the row wins (lowest CSR-by-target slot).
+ *                          win (optional, MAX only, training): winner masks, 16 bytes per CSR-by-target position p =
+ *                          4 uint32 words; bit (c % 32) of word (c / 32) is set when channel c of the row's target took its
+ *                          max from position p.  Every position is written (all-zero masks included).
  *   pcc_gnn_fc1_pool_fwd : fc1 + act + bn3 statistics + global_mean_pool (:87-92): psum[B,256] = per-graph sums of
  *                          act(fc1(h)), partials [nblk][2][256]; the per-node [M,256] tensor never reaches HBM. */
 int64_t pcc_gnn_packed_bytes(void);
 int pcc_gnn_max_blocks(void);
 int pcc_gnn_pack_weights(const float* w_rel2, const float* w_root2, const float* w_fc1, void* packed, int device, void* stream);
-int pcc_gnn_conv1_fwd(const float* x, int F, const int64_t* rowptr, const int32_t* col, const float* w, int mean,
+int pcc_gnn_conv1_fwd(const float* x, int F, const int64_t* rowptr, const int32_t* col, const float* w, int aggr,
                       const float* w_rel, const float* w_root, const float* bias, int64_t M, int act, float* agg_out,
                       float* z_out, float* partials, int* nblk_out, int device, void* stream);
 int pcc_gnn_bn_finalize(const float* partials, int nblk, int Cn, int64_t rows, const float* gamma, const float* beta,
@@ -258,9 +269,9 @@ int pcc_gnn_bn_eval(const float* running_mean, const float* running_var, const f
                     int Cn, float* scale, float* shift, int device, void* stream);
 int pcc_gnn_bn_apply(const float* z, const float* scale, const float* shift, int64_t M, int act, void* h_bf16, int device,
                      void* stream);
-int pcc_gnn_conv_fwd(const void* h_in_bf16, const int64_t* rowptr, const int32_t* col, const float* w, int mean,
+int pcc_gnn_conv_fwd(const void* h_in_bf16, const int64_t* rowptr, const int32_t* col, const float* w, int aggr,
                      const void* packed, const float* bias, int64_t M, int act, void* agg_out_bf16, float* z_out,
-                     float* partials, const int64_t* membership, float* psum, int64_t B, int* nblk_out, int device,
+                     float* partials, const int64_t* membership, float* psum, int64_t B, void* win, int* nblk_out, int device,
                      void* stream);
 /* graph-sized glue of the pooled outputs: P = psum / max(n_g, 1), y = P * scale + shift (mean pool commuted with the affine) */
 int pcc_gnn_pool_affine(const float* psum, const int64_t* counts, const float* scale, const float* shift, int64_t B, int Cn,
@@ -281,7 +292,9 @@ int pcc_gnn_fc1_pool_fwd(const void* h_in_bf16, const void* packed, const float*
  *                             the same row for every node of a graph: mean pooling straight after the block); dagg_out | droot_out (bf16) = dz [W_rel | W_root];
  *                             dw_part [nblk][128][256] = dz^T [agg | h_in] accumulated in TMEM; db_part [nblk][128].
  *   pcc_gnn_agg_bwd         : dh_inout[j] += sum_{e: src(e)=j} w_e dagg[dst(e)] (CSR by source) + the bn sums of the
- *                             previous block (z_prev, its mean / invstd).
+ *                             previous block (z_prev, its mean / invstd).  ADD / MEAN: w_src carries 1/deg(dst) for mean.
+ *                             MAX: only the channels edge e won count, win[pos_src[q]] (.) dagg[dst(e)], pos_src[E] =
+ *                             CSR-by-target position of every by-source entry q, win = the masks of pcc_gnn_conv_fwd.
  *   pcc_gnn_conv1_bwd       : partials [nblk][128][2F+1] = (dW_rel | dW_root | db) of GraphConv 1. */
 /* backward of the same glue from G = dL/dy [B, Cn]: gs = G f / n_g, kap = f sum(G) / M, lam = f sum(G xhat(P)) / M,
  * dgamma = sum(G xhat), dbeta = sum(G)   (f = s, or 1 with use_scale = 0) */
@@ -299,9 +312,9 @@ int pcc_gnn_conv_bwd(const void* dh_bf16, const int64_t* membership, const float
                      const float* bn_c1, const float* bn_c2, const void* agg_bf16, const void* h_in_bf16, const void* packed,
                      int64_t M, int act, void* dagg_out_bf16, void* droot_out_bf16, float* dw_part, float* db_part, int* nblk_out,
                      int device, void* stream);
-int pcc_gnn_agg_bwd(const void* dagg_bf16, const int64_t* rowptr_src, const int32_t* col_src, const float* w_src,
-                    void* dh_inout_bf16, const float* z_prev, const float* mu_prev, const float* r_prev, int64_t M, int act,
-                    float* partials, int* nblk_out, int device, void* stream);
+int pcc_gnn_agg_bwd(const void* dagg_bf16, const int64_t* rowptr_src, const int32_t* col_src, const float* w_src, int aggr,
+                    const int32_t* pos_src, const void* win, void* dh_inout_bf16, const float* z_prev, const float* mu_prev,
+                    const float* r_prev, int64_t M, int act, float* partials, int* nblk_out, int device, void* stream);
 int pcc_gnn_conv1_bwd(const void* dh_bf16, const float* z, const float* bn_mean, const float* bn_invstd, const float* bn_scale,
                       const float* bn_c1, const float* bn_c2, const float* agg, const float* x, int F, int64_t M, int act,
                       float* partials, int* nblk_out, int device, void* stream);

@@ -39,8 +39,10 @@ __global__ void gnn_pack_kernel(const float* __restrict__ w_rel, const float* __
 // floats per row, independent loads -> deep memory-level parallelism, no shuffles), aggregate and own row parked in
 // shared memory.  (B) warp = 32 of those nodes in turn, lane = output channels lane + 32 j: z = b + W_rel agg + W_root x
 // from broadcast shared-memory reads, coalesced 128-byte stores of z1, per-lane column sums of act(z1), act(z1)^2
-// (BatchNorm statistics).  Writes agg1 (kept for the weight gradient).
-template <int ACT, int FP>
+// (BatchNorm statistics).  Writes agg1 (kept for the weight gradient).  MAX: the aggregate is the max of the fp32 products
+// w_e x[src(e)] (0 for a node without in-edges); conv1 needs no winners (x takes no gradient, the weight gradient reads
+// agg1).
+template <int ACT, int FP, bool MAX>
 __global__ void __launch_bounds__(256) gnn_conv1_fwd_kernel(const float* __restrict__ x, int F, GnnGraph g,
                                                             const float* __restrict__ w_rel, const float* __restrict__ w_root,
                                                             const float* __restrict__ bias, int64_t M, float* __restrict__ agg_out,
@@ -69,15 +71,24 @@ __global__ void __launch_bounds__(256) gnn_conv1_fwd_kernel(const float* __restr
     for (int f = 0; f < FP; ++f) a[f] = xs[f] = 0.f;
     if (node < M) {
       const int64_t pb = __ldg(g.rowptr + node), pe = __ldg(g.rowptr + node + 1);
+      if (MAX) {
+#pragma unroll
+        for (int f = 0; f < FP; ++f) a[f] = -INFINITY;
+      }
 #pragma unroll 4
       for (int64_t p = pb; p < pe; ++p) {
         const int64_t sidx = (int64_t)__ldg(g.col + p);
         const float we = g.w ? __ldg(g.w + p) : 1.f;
 #pragma unroll
         for (int f = 0; f < FP; ++f)
-          if (f < F) a[f] = fmaf(we, __ldg(x + sidx * F + f), a[f]);
+          if (f < F) a[f] = MAX ? fmaxf(a[f], __fmul_rn(we, __ldg(x + sidx * F + f))) : fmaf(we, __ldg(x + sidx * F + f), a[f]);
       }
-      const float inv = (g.mean && pe > pb) ? 1.f / (float)(pe - pb) : 1.f;
+      if (MAX) {
+#pragma unroll
+        for (int f = 0; f < FP; ++f)
+          if (f >= F || pe == pb) a[f] = 0.f;   // (the padded inputs meet zero weights in phase B: they must be finite)
+      }
+      const float inv = (!MAX && g.aggr == PCC_POOL_MEAN && pe > pb) ? 1.f / (float)(pe - pb) : 1.f;
 #pragma unroll
       for (int f = 0; f < FP; ++f) {
         a[f] *= inv;
@@ -243,9 +254,13 @@ struct ConvFwdParams {
   const int64_t* membership;   // optional (with psum): graph of every node
   float* psum;                 // optional [B,C]: per-graph sums of act(z) (global_mean_pool straight after the block)
   int64_t M, num_tiles;
+  uint4* win;                  // MAX, optional [E]: winner mask of every CSR-by-target position (training)
 };
 
-template <int ACT>
+// MAX: the gather warps reduce with compare / select (slot_max) instead of the packed adds and keep, per lane and
+// channel, the max and the position of its winner inside the node's row; with p.win they also write the node's winner
+// masks (write_win_masks, in the first 512 bytes of the warp's gather slot, which is idle between two nodes).
+template <int ACT, bool MAX>
 __global__ void __launch_bounds__(kConvThreads, 1) gnn_conv_fwd_kernel(const ConvFwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* Aimg = smem;                       // 64 KB (single buffer: the MMA of a tile takes ~0.5k cycles, its gather >10k)
@@ -306,7 +321,10 @@ __global__ void __launch_bounds__(kConvThreads, 1) gnn_conv_fwd_kernel(const Con
         const int r = warp + kLoadWarps * i;
         const bool ok = n0 + r < p.M;
         float acc[4] = {0.f, 0.f, 0.f, 0.f};
+        int arg[4] = {0, 0, 0, 0};
+        if (MAX) acc[0] = acc[1] = acc[2] = acc[3] = -INFINITY;
         const int64_t deg = pe - pb;
+        const int64_t row0 = pb;
         // root row of the node: issued early, used last
         uint2 root = make_uint2(0u, 0u);
         if (ok) root = __ldg(reinterpret_cast<const uint2*>(hin + (size_t)(n0 + r) * kRowB) + lane);
@@ -337,12 +355,19 @@ __global__ void __launch_bounds__(kConvThreads, 1) gnn_conv_fwd_kernel(const Con
           if (ccnt > 0) {
             mbar_wait_b(bar, gphase);
             gphase ^= 1;
-            slot_reduce<(int)kRowB>(slot, ccnt, lane, p.g.w != nullptr, cw, acc);
+            if (MAX) slot_max<(int)kRowB>(slot, ccnt, lane, p.g.w != nullptr, cw, (int)(done - ccnt), acc, arg);
+            else slot_reduce<(int)kRowB>(slot, ccnt, lane, p.g.w != nullptr, cw, acc);
             __syncwarp();   // every lane has read the slot before the next chunk's copies overwrite it
           }
           if (next_node) { pb = npb; pe = npe; break; }
         }
-        if (p.g.mean && deg > 0) {
+        if (MAX) {
+          if (deg == 0) acc[0] = acc[1] = acc[2] = acc[3] = 0.f;
+          if (p.win != nullptr && deg > 0) {
+            write_win_masks(reinterpret_cast<uint4*>(slot), p.win + row0, (int)deg, lane, arg);
+            fence_proxy_async();   // the generic writes to the slot are ordered before the next node's bulk copies into it
+          }
+        } else if (p.g.aggr == PCC_POOL_MEAN && deg > 0) {
           const float inv = 1.f / (float)deg;
           acc[0] *= inv; acc[1] *= inv; acc[2] *= inv; acc[3] *= inv;
         }
@@ -654,15 +679,21 @@ extern "C" int pcc_gnn_pack_weights(const float* w_rel2, const float* w_root2, c
   return check_launch(__func__);
 }
 
-extern "C" int pcc_gnn_conv1_fwd(const float* x, int F, const int64_t* rowptr, const int32_t* col, const float* w, int mean,
+#define GNN_AGGR_CHECK(aggr) \
+  PCC_REQUIRE(aggr == PCC_POOL_ADD || aggr == PCC_POOL_MEAN || aggr == PCC_POOL_MAX, "aggr must be PCC_POOL_ADD / MEAN / MAX")
+
+extern "C" int pcc_gnn_conv1_fwd(const float* x, int F, const int64_t* rowptr, const int32_t* col, const float* w, int aggr,
                                  const float* w_rel, const float* w_root, const float* bias, int64_t M, int act, float* agg_out,
                                  float* z_out, float* partials, int* nblk_out, int device, void* stream) {
   PCC_ENTER(device);
   PCC_REQUIRE(F >= 1 && F <= 8, "fused conv1 needs input_dim <= 8");
+  GNN_AGGR_CHECK(aggr);
   int blocks = 1;
-  GnnGraph g{rowptr, col, w, mean};
+  GnnGraph g{rowptr, col, w, aggr};
+  const bool mx = aggr == PCC_POOL_MAX;
   GNN_ACT_DISPATCH(act, {
-    auto kern = F <= 4 ? gnn_conv1_fwd_kernel<A, 4> : gnn_conv1_fwd_kernel<A, 8>;
+    auto kern = mx ? (F <= 4 ? gnn_conv1_fwd_kernel<A, 4, true> : gnn_conv1_fwd_kernel<A, 8, true>)
+                   : (F <= 4 ? gnn_conv1_fwd_kernel<A, 4, false> : gnn_conv1_fwd_kernel<A, 8, false>);
     blocks = (int)(cdiv(M, 256) < 592 ? cdiv(M, 256) : 592);   // (measured: 592 blocks 52 us, one resident wave of 444 57 us)
     if (blocks < 1) blocks = 1;
     PCC_K(kern)<<<blocks, 256, 0, (cudaStream_t)stream>>>(x, F, g, w_rel, w_root, bias, M, agg_out, z_out, partials);
@@ -708,18 +739,21 @@ extern "C" int pcc_gnn_bn_apply(const float* z, const float* scale, const float*
   return check_launch(__func__);
 }
 
-extern "C" int pcc_gnn_conv_fwd(const void* h_in_bf16, const int64_t* rowptr, const int32_t* col, const float* w, int mean,
+extern "C" int pcc_gnn_conv_fwd(const void* h_in_bf16, const int64_t* rowptr, const int32_t* col, const float* w, int aggr,
                                 const void* packed, const float* bias, int64_t M, int act, void* agg_out_bf16, float* z_out,
-                                float* partials, const int64_t* membership, float* psum, int64_t B, int* nblk_out, int device,
-                                void* stream) {
+                                float* partials, const int64_t* membership, float* psum, int64_t B, void* win, int* nblk_out,
+                                int device, void* stream) {
   PCC_ENTER(device);
   PCC_REQUIRE(psum == nullptr || membership != nullptr, "psum needs the membership vector");
+  GNN_AGGR_CHECK(aggr);
+  PCC_REQUIRE(win == nullptr || aggr == PCC_POOL_MAX, "winner masks belong to max aggregation");
   if (psum) PCC_CUDA(cudaMemsetAsync(psum, 0, (size_t)B * kC * sizeof(float), (cudaStream_t)stream));
   ConvFwdParams p{};
   p.membership = membership;
   p.psum = psum;
   p.h_in = (const __nv_bfloat16*)h_in_bf16;
-  p.g = GnnGraph{rowptr, col, w, mean};
+  p.g = GnnGraph{rowptr, col, w, aggr};
+  p.win = (uint4*)win;
   p.wimg = (const uint8_t*)packed;
   p.bias = bias;
   p.agg_out = (__nv_bfloat16*)agg_out_bf16;
@@ -734,7 +768,7 @@ extern "C" int pcc_gnn_conv_fwd(const void* h_in_bf16, const int64_t* rowptr, co
   {
     ProfScope prof(3, (cudaStream_t)stream);
     GNN_ACT_DISPATCH(act, {
-      auto kern = gnn_conv_fwd_kernel<A>;
+      auto kern = aggr == PCC_POOL_MAX ? gnn_conv_fwd_kernel<A, true> : gnn_conv_fwd_kernel<A, false>;
       PCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
       PCC_K(kern)<<<grid, kConvThreads, smem_bytes, (cudaStream_t)stream>>>(p);
     });

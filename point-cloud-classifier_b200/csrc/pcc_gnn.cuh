@@ -99,6 +99,81 @@ __device__ __forceinline__ void slot_reduce(const uint8_t* slot, int cnt, int la
   f32x2_unpack(a23, acc[2], acc[3]);
 }
 
+// ---- max aggregation (conv forward): per channel the running max of w_u * row_u (the product in fp32, as
+// GraphConv.message) and the row position of its winner, `base + u` (base = rows of the node taken in earlier gather
+// rounds).  The strict > keeps the first of equal values: the winner is the lowest CSR-by-target position.
+template <int ROWB>
+__device__ __forceinline__ void slot_max(const uint8_t* slot, int cnt, int lane, bool weighted, float cw, int base,
+                                         float (&mx)[4], int (&arg)[4]) {
+  const uint8_t* p = slot + lane * 8;
+  if (!weighted) {
+#pragma unroll 2
+    for (int u = 0; u < cnt; ++u) {
+      const uint2 v = *reinterpret_cast<const uint2*>(p + u * ROWB);
+      const float m[4] = {bf16_lo(v.x), bf16_hi(v.x), bf16_lo(v.y), bf16_hi(v.y)};
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (m[j] > mx[j]) { mx[j] = m[j]; arg[j] = base + u; }
+    }
+  } else {
+#pragma unroll 2
+    for (int u = 0; u < cnt; ++u) {
+      const uint2 v = *reinterpret_cast<const uint2*>(p + u * ROWB);
+      const float wu = __shfl_sync(0xffffffffu, cw, u);
+      const float m[4] = {__fmul_rn(wu, bf16_lo(v.x)), __fmul_rn(wu, bf16_hi(v.x)), __fmul_rn(wu, bf16_lo(v.y)),
+                          __fmul_rn(wu, bf16_hi(v.y))};
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (m[j] > mx[j]) { mx[j] = m[j]; arg[j] = base + u; }
+    }
+  }
+}
+
+// Winner masks of one node (layout: include/pcc.h, pcc_gnn_conv_fwd): position s of the node's row gets 16 bytes, bit
+// c % 32 of word c / 32 set when channel c's max came from s.  Lane l owns channels 4l .. 4l+3 = bits 4 (l & 7) ..
+// +3 of word l >> 3.  Built 32 positions at a time in `scratch` (32 x 16 B of shared memory) with one shared atomicOr
+// per lane and channel, then stored coalesced; every position of the row is written, all-zero masks included.
+__device__ __forceinline__ void write_win_masks(uint4* scratch, uint4* __restrict__ win_row, int deg, int lane,
+                                                const int (&arg)[4]) {
+  uint32_t* word = reinterpret_cast<uint32_t*>(scratch) + (lane >> 3);
+  const int sh = 4 * (lane & 7);
+  for (int s0 = 0; s0 < deg; s0 += 32) {
+    scratch[lane] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int r = arg[j] - s0;
+      if (r >= 0 && r < 32) atomicOr(word + 4 * r, 1u << (sh + j));
+    }
+    __syncwarp();
+    if (s0 + lane < deg) win_row[s0 + lane] = scratch[lane];
+    __syncwarp();
+  }
+}
+
+// ---- max aggregation backward: the landed dagg rows times the edge weight, each channel only where the slot's winner
+// mask (16 bytes per row in `masks`, landed with the rows) has its bit.  One fp32 FMA chain per channel pair, in row
+// order: deterministic.
+template <int ROWB>
+__device__ __forceinline__ void slot_reduce_masked(const uint8_t* slot, const uint8_t* masks, int cnt, int lane, bool weighted,
+                                                   float cw, float (&acc)[4]) {
+  uint64_t a01 = f32x2(acc[0], acc[1]), a23 = f32x2(acc[2], acc[3]);
+  const uint8_t* p = slot + lane * 8;
+  const uint32_t* mw = reinterpret_cast<const uint32_t*>(masks) + (lane >> 3);
+  const int sh = 4 * (lane & 7);
+#pragma unroll 2
+  for (int u = 0; u < cnt; ++u) {
+    const uint2 v = *reinterpret_cast<const uint2*>(p + u * ROWB);
+    const uint32_t b = mw[4 * u] >> sh;
+    const float wu = weighted ? __shfl_sync(0xffffffffu, cw, u) : 1.f;
+    const uint64_t w01 = f32x2((b & 1u) ? wu : 0.f, (b & 2u) ? wu : 0.f);
+    const uint64_t w23 = f32x2((b & 4u) ? wu : 0.f, (b & 8u) ? wu : 0.f);
+    a01 = ffma2(w01, bf16x2_to_f32x2(v.x), a01); a23 = ffma2(w23, bf16x2_to_f32x2(v.y), a23);
+  }
+  f32x2_unpack(a01, acc[0], acc[1]);
+  f32x2_unpack(a23, acc[2], acc[3]);
+}
+
 // bounded mbarrier wait: a protocol bug traps instead of hanging the GPU.  The clock is read once per 1024 failed
 // polls only: with a clock read in every iteration the wait loops were 15 % of ALL instructions the conv forward kernel
 // executed (ncu, profiles/r2/ncu_gnn_r2e.txt) — issue slots taken from the warps that had work.
@@ -192,7 +267,7 @@ struct GnnGraph {
   const int64_t* rowptr;   // [M+1] CSR by target (forward) or by source (backward)
   const int32_t* col;      // [E] neighbour node per CSR slot
   const float* w;          // [E] edge weight per CSR slot, or null
-  int mean;                // forward: divide the aggregate by the in-degree
+  int aggr;                // forward: PCC_POOL_ADD / MEAN (divide by the in-degree) / MAX
 };
 
 }  // namespace gnn

@@ -609,17 +609,22 @@ __global__ void __launch_bounds__(kCbThreads, 1) gnn_conv_bwd_kernel(const ConvB
 // sum dh xhat of the PREVIOUS block (z_prev, its mean / invstd) per block.
 // The neighbour rows (256 B of bf16) are fetched by the TMA engine into a per-warp shared-memory slot (one
 // cp.async.bulk per row, all of a node's rows in flight at once, no registers tied up), like the forward gather.
+// MAX: dh[j] = droot[j] + sum_{q in row j} w_q (win[pos[q]] (.) dagg[col[q]]): the 16-byte winner mask of every slot's
+// CSR-by-target position pos[q] lands next to its row (a second bulk copy on the same mbarrier) and masks the channels.
 constexpr int kAggSlotRows = 22;
 constexpr uint32_t kAggRowB = kC * 2, kAggSlotB = kAggSlotRows * kAggRowB;
-template <int ACT>
+constexpr uint32_t kAggMaskB = 16, kAggMaskSlotB = kAggSlotRows * kAggMaskB;
+template <int ACT, bool MAX>
 __global__ void __launch_bounds__(256, 3) gnn_agg_bwd_kernel(const __nv_bfloat16* __restrict__ dagg, GnnGraph g, __nv_bfloat16* __restrict__ dh,
                                                           const float* __restrict__ z_prev, const float* __restrict__ mu_prev,
-                                                          const float* __restrict__ r_prev, int64_t M, float* __restrict__ partials) {
+                                                          const float* __restrict__ r_prev, int64_t M, float* __restrict__ partials,
+                                                          const int32_t* __restrict__ pos, const uint8_t* __restrict__ win) {
   extern __shared__ __align__(128) uint8_t smem_agg[];
   uint8_t* slots = smem_agg;                                                // [8 warps][22 rows][256 B]
   float* red = reinterpret_cast<float*>(smem_agg + 8 * kAggSlotB);          // [8][2][C]
   uint64_t* gbar = reinterpret_cast<uint64_t*>(red + 8 * 2 * kC);           // [8]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  uint8_t* mslot = reinterpret_cast<uint8_t*>(gbar + 8) + warp * kAggMaskSlotB;   // MAX: [8 warps][22 rows][16 B]
   if (threadIdx.x < 8) mbar_init(&gbar[threadIdx.x], 1);
   fence_mbar_init();
   __syncthreads();
@@ -640,6 +645,7 @@ __global__ void __launch_bounds__(256, 3) gnn_agg_bwd_kernel(const __nv_bfloat16
   int cnt = (pe - pb < kAggSlotRows) ? pe - pb : kAggSlotRows;
   int myc = lane < cnt ? __ldg(g.col + pb + lane) : 0;
   float myw = (g.w && lane < cnt) ? __ldg(g.w + pb + lane) : 1.f;
+  int myq = (MAX && lane < cnt) ? __ldg(pos + pb + lane) : 0;
   uint2 dh_next = make_uint2(0u, 0u);
   float4 z_next = make_float4(0.f, 0.f, 0.f, 0.f);
   if (node < M) {
@@ -662,9 +668,12 @@ __global__ void __launch_bounds__(256, 3) gnn_agg_bwd_kernel(const __nv_bfloat16
     int done = 0;
     for (;;) {
       if (cnt > 0) {
-        if (lane == 0) mbar_arrive_expect_tx(bar, (uint32_t)cnt * kAggRowB);
+        if (lane == 0) mbar_arrive_expect_tx(bar, (uint32_t)cnt * (MAX ? kAggRowB + kAggMaskB : kAggRowB));
         __syncwarp();
-        if (lane < cnt) bulk_g2s(slot + lane * kAggRowB, src + (size_t)myc * kAggRowB, kAggRowB, bar);
+        if (lane < cnt) {
+          bulk_g2s(slot + lane * kAggRowB, src + (size_t)myc * kAggRowB, kAggRowB, bar);
+          if (MAX) bulk_g2s(mslot + lane * kAggMaskB, win + (size_t)myq * kAggMaskB, kAggMaskB, bar);
+        }
       }
       const int ccnt = cnt;
       const float cw = myw;
@@ -674,6 +683,7 @@ __global__ void __launch_bounds__(256, 3) gnn_agg_bwd_kernel(const __nv_bfloat16
       cnt = (npe - npb < kAggSlotRows) ? npe - npb : kAggSlotRows;
       myc = lane < cnt ? __ldg(g.col + npb + lane) : 0;
       myw = (g.w && lane < cnt) ? __ldg(g.w + npb + lane) : 1.f;
+      if (MAX) myq = lane < cnt ? __ldg(pos + npb + lane) : 0;
       if (first) {
         acc[0] = bf16_lo(acc0.x); acc[1] = bf16_hi(acc0.x); acc[2] = bf16_lo(acc0.y); acc[3] = bf16_hi(acc0.y);
         first = false;
@@ -681,7 +691,8 @@ __global__ void __launch_bounds__(256, 3) gnn_agg_bwd_kernel(const __nv_bfloat16
       if (ccnt > 0) {
         mbar_wait_b(bar, gphase);
         gphase ^= 1;
-        slot_reduce<(int)kAggRowB>(slot, ccnt, lane, g.w != nullptr, cw, acc);
+        if (MAX) slot_reduce_masked<(int)kAggRowB>(slot, mslot, ccnt, lane, g.w != nullptr, cw, acc);
+        else slot_reduce<(int)kAggRowB>(slot, ccnt, lane, g.w != nullptr, cw, acc);
         __syncwarp();
       }
       if (next_node) { pb = nb; pe = ne; nb = n2b; ne = n2e; break; }
@@ -874,21 +885,25 @@ extern "C" int pcc_gnn_conv_bwd(const void* dh_bf16, const int64_t* membership, 
 }
 
 extern "C" int pcc_gnn_agg_bwd(const void* dagg_bf16, const int64_t* rowptr_src, const int32_t* col_src, const float* w_src,
-                               void* dh_inout_bf16, const float* z_prev, const float* mu_prev, const float* r_prev, int64_t M,
-                               int act, float* partials, int* nblk_out, int device, void* stream) {
+                               int aggr, const int32_t* pos_src, const void* win, void* dh_inout_bf16, const float* z_prev,
+                               const float* mu_prev, const float* r_prev, int64_t M, int act, float* partials, int* nblk_out,
+                               int device, void* stream) {
   PCC_ENTER(device);
+  PCC_REQUIRE(aggr == PCC_POOL_ADD || aggr == PCC_POOL_MEAN || aggr == PCC_POOL_MAX, "aggr must be PCC_POOL_ADD / MEAN / MAX");
+  const bool mx = aggr == PCC_POOL_MAX;
+  PCC_REQUIRE(!mx || (pos_src != nullptr && win != nullptr), "max aggregation needs pos_src and the winner masks");
   int blocks = 1;
-  GnnGraph g{rowptr_src, col_src, w_src, 0};
+  GnnGraph g{rowptr_src, col_src, w_src, aggr};
   {
     ProfScope prof(5, (cudaStream_t)stream);
-    const int smem_bytes = 8 * kAggSlotB + 8 * 2 * kC * 4 + 64;
+    const int smem_bytes = 8 * kAggSlotB + 8 * 2 * kC * 4 + 64 + (mx ? 8 * (int)kAggMaskSlotB : 0);
     GNN_ACT_DISPATCH(act, {
-      auto kern = gnn_agg_bwd_kernel<A>;
+      auto kern = mx ? gnn_agg_bwd_kernel<A, true> : gnn_agg_bwd_kernel<A, false>;
       PCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
       blocks = gnn_resident_blocks((const void*)kern, 256, smem_bytes, cdiv(M, 8));
       *nblk_out = blocks;
       PCC_K(kern)<<<blocks, 256, smem_bytes, (cudaStream_t)stream>>>((const __nv_bfloat16*)dagg_bf16, g, (__nv_bfloat16*)dh_inout_bf16, z_prev, mu_prev,
-                                                                     r_prev, M, partials);
+                                                                     r_prev, M, partials, pos_src, (const uint8_t*)win);
     });
   }
   return check_launch(__func__);

@@ -240,6 +240,25 @@ __global__ void __launch_bounds__(kCsrtBlkThreads, 1) csrt_block_kernel(const in
   }
 }
 
+// ---- by-target position of every by-source entry of such a graph (max aggregation's backward reads the winner mask
+// of an edge at its CSR-by-target position).  Thread = by-target slot p = (target t = p / k, source j = col_d[p]); the
+// entry (j -> t) of the by-source CSR is the unique t in j's row (ascending targets, simple graph): a binary search.
+__global__ void csrt_pos_kernel(const int32_t* __restrict__ col_d, int k, int64_t E, const int64_t* __restrict__ rowptr_s,
+                                const int32_t* __restrict__ col_s, int32_t* __restrict__ pos_s) {
+  const int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (p >= E) return;
+  const int j = __ldg(col_d + p);
+  const int t = (int)(p / k);
+  int64_t lo = __ldg(rowptr_s + j), hi = __ldg(rowptr_s + j + 1);
+  const int64_t end = hi;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (__ldg(col_s + mid) < t) lo = mid + 1; else hi = mid;
+  }
+  if (lo >= end || __ldg(col_s + lo) != t) __trap();   // not the transpose of col_d
+  pos_s[lo] = (int32_t)p;
+}
+
 // ------------------------------------------------------------------ aggregation
 // tpn threads per node, each owning float4 channel groups c = 4*(lane + it*tpn)
 template <bool VEC4>
@@ -542,6 +561,17 @@ extern "C" int pcc_csr_transpose_blocks(const int32_t* col_d, int k, const int64
   }
   PCC_CUDA(cudaFuncSetAttribute(csrt_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCsrtBlkSmem));
   PCC_K(csrt_block_kernel)<<<(unsigned)B, kCsrtBlkThreads, kCsrtBlkSmem, (cudaStream_t)stream>>>(col_d, k, offsets, n, rowptr_s, col_s);
+  return check_launch(__func__);
+}
+
+extern "C" int pcc_csr_transpose_pos(const int32_t* col_d, int k, int64_t n, const int64_t* rowptr_s, const int32_t* col_s,
+                                     int32_t* pos_s, int device, void* stream) {
+  PCC_ENTER(device);
+  PCC_REQUIRE(k >= 1, "k must be positive");
+  PCC_REQUIRE(n * (int64_t)k < (int64_t)0x7fffffff, "edge count exceeds int32 range");
+  const int64_t E = n * (int64_t)k;
+  if (E == 0) return 0;
+  PCC_K(csrt_pos_kernel)<<<(unsigned)cdiv(E, 256), 256, 0, (cudaStream_t)stream>>>(col_d, k, E, rowptr_s, col_s, pos_s);
   return check_launch(__func__);
 }
 

@@ -53,6 +53,7 @@ _SIGS = {
     "pcc_csr_build": [_vp, _i64, _i64, _vp, _vp, _vp, _i32, _vp],
     "pcc_csr_transpose": [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _i32, _vp],
     "pcc_csr_transpose_blocks": [_vp, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _vp],
+    "pcc_csr_transpose_pos": [_vp, _i32, _i64, _vp, _vp, _vp, _i32, _vp],
     "pcc_graph_aggregate_fwd": [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _i32, _vp],
     "pcc_graph_aggregate_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _i32, _vp],
     "pcc_knn": [_vp, _i64, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _i32, _vp],
@@ -80,7 +81,7 @@ _SIGS = {
     "pcc_gnn_bn_finalize": [_vp, _i32, _i32, _i64, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp],
     "pcc_gnn_bn_eval": [_vp, _vp, _vp, _vp, _f32, _i32, _vp, _vp, _i32, _vp],
     "pcc_gnn_bn_apply": [_vp, _vp, _vp, _i64, _i32, _vp, _i32, _vp],
-    "pcc_gnn_conv_fwd": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i64, C.POINTER(C.c_int), _i32, _vp],
+    "pcc_gnn_conv_fwd": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp, C.POINTER(C.c_int), _i32, _vp],
     "pcc_gnn_fc1_pool_fwd": [_vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, C.POINTER(C.c_int), _i32, _vp],
     "pcc_gnn_pool_affine": [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _i32, _vp],
     "pcc_gnn_pool_bwd_prep": [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp],
@@ -88,7 +89,7 @@ _SIGS = {
     "pcc_gnn_reduce": [_vp, _i32, _i64, _vp, _i32, _vp],
     "pcc_gnn_fc1_bwd": [_vp] * 12 + [_i64, _i32, _vp, _vp, _vp, _vp, C.POINTER(C.c_int), _i32, _vp],
     "pcc_gnn_conv_bwd": [_vp] * 12 + [_i64, _i32, _vp, _vp, _vp, _vp, C.POINTER(C.c_int), _i32, _vp],
-    "pcc_gnn_agg_bwd": [_vp] * 8 + [_i64, _i32, _vp, C.POINTER(C.c_int), _i32, _vp],
+    "pcc_gnn_agg_bwd": [_vp, _vp, _vp, _vp, _i32] + [_vp] * 6 + [_i64, _i32, _vp, C.POINTER(C.c_int), _i32, _vp],
     "pcc_gnn_conv1_bwd": [_vp] * 9 + [_i32, _i64, _i32, _vp, C.POINTER(C.c_int), _i32, _vp],
     "pcc_launch_count": [_i32],
     "pcc_prof_enable": [_i32],

@@ -5,8 +5,15 @@ accumulation, fp32 pre-activations and BatchNorm statistics.  Stated tolerance: 
 
 Supported: hidden_dim 128 or 64 (64 runs the 128-wide kernels on zero-padded parameters: padded channels stay exactly 0
 through conv / act / BatchNorm), deepchem_style True (fc1 per node, then mean pool) and False (mean pool straight after
-conv2; fc1 / bn3 / fc2 then run on [B, .] tensors through the layer-wise ops), local_pooling add / mean, input_dim <= 8,
-tanh / relu / gelu (configs/graph_net.yaml is inside).  hidden_dim 256 and max aggregation take the fp32 layer-wise path.
+conv2; fc1 / bn3 / fc2 then run on [B, .] tensors through the layer-wise ops), local_pooling add / mean / max,
+input_dim <= 8, tanh / relu / gelu (configs/graph_net.yaml is inside).  hidden_dim 256 takes the fp32 layer-wise path.
+
+Max aggregation: agg_i[c] = max_{e: dst(e)=i} w_e h[src(e)][c] (the product in fp32), 0 for a node without in-edges.
+Ties go to the FIRST edge: the lowest position in the target's CSR-by-target row (the lowest edge id of an edge list,
+the kNN slot order of a neighbour table), and the whole gradient of agg_i[c] goes to that edge.  In this mode h1 is
+bf16, so exact ties between neighbours are common; the fp32 path applies the same rule.  Training writes one 16-byte
+winner mask per edge in the conv2 forward (pcc_gnn_conv_fwd) that the aggregation backward reads at the edge's
+CSR-by-target position (FusedGraph.by_src).
 """
 from __future__ import annotations
 
@@ -22,12 +29,13 @@ C_HID, C_FC = 128, 256
 
 
 def supported(input_dim: int, hidden_dim: int, act: str, aggr: str, deepchem: bool) -> bool:
-    return hidden_dim in (64, C_HID) and aggr in ("add", "mean") and 1 <= input_dim <= 8 and act in ("tanh", "relu", "gelu")
+    return hidden_dim in (64, C_HID) and aggr in ("add", "mean", "max") and 1 <= input_dim <= 8 and act in ("tanh", "relu", "gelu")
 
 
 class FusedGraph:
     """CSR views of a batched edge list in the layout the fused kernels read: rowptr int64 [n+1], col int32 [E]
-    (neighbour node per slot), w fp32 [E] or None.  by_dst feeds the forward aggregation, by_src its transpose."""
+    (neighbour node per slot), w fp32 [E] or None.  by_dst feeds the forward aggregation, by_src its transpose (for max
+    aggregation with the CSR-by-target position of every by-source entry)."""
 
     def __init__(self, edges: Optional[torch.Tensor], n: int, weights: Optional[torch.Tensor], aggr: str, by_dst=None, k_uniform: int = 0,
                  block_offsets: Optional[torch.Tensor] = None):
@@ -45,17 +53,19 @@ class FusedGraph:
         if by_dst is not None:                       # e.g. a kNN graph: k consecutive edges per target, already grouped
             self.rowptr_d, self.col_d = by_dst
             self.w_d = weights
-            perm_d = None
+            perm_d = None                            # slot p of by_dst is edge p
         else:
             csr = GraphCSR(edges, n)
             self.rowptr_d, perm_d = csr.by_dst
             pl = perm_d.long()
             self.col_d = edges[0][pl].to(torch.int32)
             self.w_d = weights[pl].contiguous() if weights is not None else None
-        self._edges, self._weights, self._csr = edges, weights, csr
+        self._edges, self._weights, self._csr, self._perm_d = edges, weights, csr, perm_d
         self._src = None
 
     def by_src(self):
+        """(rowptr_s int64 [n+1], col_s int32 [E] = target per slot, w_s fp32 [E] or None, pos_s): w_s folds 1 / deg(target)
+        for mean; pos_s (max only, else None) int32 [E] = the CSR-by-target position of every by-source entry."""
         if self._src is None and self._weights is None and self.block_offsets is not None and self.k_uniform > 0:
             # kNN graph: per-cloud transpose in shared memory (pcc_csr_transpose_blocks); mean folds 1 / deg = 1 / k
             dev = L.require_cuda(self.col_d, self.block_offsets)
@@ -63,10 +73,14 @@ class FusedGraph:
             col_s = torch.empty(max(self.E, 1), dtype=torch.int32, device=self.col_d.device)
             call("pcc_csr_transpose_blocks", ptr(self.col_d), int(self.k_uniform), ptr(self.block_offsets),
                  self.block_offsets.numel() - 1, self.n, ptr(rowptr_s), ptr(col_s), dev, L.stream_ptr(dev))
-            w_s = None
+            w_s = pos_s = None
             if self.aggr == "mean":
                 w_s = torch.full((max(self.E, 1),), 1.0 / self.k_uniform, dtype=torch.float32, device=self.col_d.device)
-            self._src = (rowptr_s, col_s, w_s)
+            if self.aggr == "max":
+                pos_s = torch.empty(max(self.E, 1), dtype=torch.int32, device=self.col_d.device)
+                call("pcc_csr_transpose_pos", ptr(self.col_d), int(self.k_uniform), self.n, ptr(rowptr_s), ptr(col_s), ptr(pos_s),
+                     dev, L.stream_ptr(dev))
+            self._src = (rowptr_s, col_s, w_s, pos_s)
         if self._src is None and self._weights is None and self.aggr == "add":
             # unweighted sum aggregation: transpose the int32 CSR directly (no edge-id permutation, no int64 index ops)
             dev = L.require_cuda(self.col_d)
@@ -75,7 +89,7 @@ class FusedGraph:
             ws = torch.empty(call("pcc_csr_workspace_bytes", self.n, self.E), dtype=torch.uint8, device=self.col_d.device)
             call("pcc_csr_transpose", ptr(self.col_d), ptr(self.rowptr_d), self.E, self.n, int(self.k_uniform), ptr(rowptr_s),
                  ptr(col_s), ptr(ws), dev, L.stream_ptr(dev))
-            self._src = (rowptr_s, col_s, None)
+            self._src = (rowptr_s, col_s, None, None)
         if self._src is None:
             from .functional import GraphCSR
             csr = self._csr or GraphCSR(self._edges, self.n)
@@ -88,7 +102,15 @@ class FusedGraph:
                 deg = (self.rowptr_d[1:] - self.rowptr_d[:-1]).clamp(min=1).to(torch.float32)
                 inv = (1.0 / deg)[dst]
                 w_s = inv if w_s is None else w_s * inv
-            self._src = (rowptr_s, col_s, w_s.contiguous() if w_s is not None else None)
+            pos_s = None
+            if self.aggr == "max":                   # by-target position of edge perm_s[q]: inv(perm_d)[perm_s[q]]
+                if self._perm_d is None:
+                    pos_s = perm_s
+                else:
+                    inv_d = torch.empty_like(self._perm_d)     # (both permutations hold max(E, 1) entries)
+                    inv_d[self._perm_d[:self.E].long()] = torch.arange(self.E, dtype=torch.int32, device=inv_d.device)
+                    pos_s = inv_d[pl] if self.E > 0 else inv_d
+            self._src = (rowptr_s, col_s, w_s.contiguous() if w_s is not None else None, pos_s)
         return self._src
 
 
@@ -107,11 +129,13 @@ def _pad(t: torch.Tensor, shape, fill: float = 0.0) -> torch.Tensor:
 
 class GraphNetFusedFn(torch.autograd.Function):
     """deepchem_style=True : (x, 14 params) -> y3[B,256] = bn3-normalised, mean-pooled act(fc1(.)) — everything before fc2.
-    deepchem_style=False: (x, 10 params) -> pooled[B,hidden] = global_mean_pool(bn2(act(conv2(.)))) — everything before fc1."""
+    deepchem_style=False: (x, 10 params) -> pooled[B,hidden] = global_mean_pool(bn2(act(conv2(.)))) — everything before fc1.
+    meta = (act, training, eps, momentum, deepchem, hidden, grad): grad = autograd was recording at the call (forward
+    itself runs without it), so that max aggregation writes its winner masks only for a step that can run a backward."""
 
     @staticmethod
     def forward(ctx, x, membership, graph: FusedGraph, counts, meta, bufs, *params):
-        act, training, eps, momentum, deepchem, Cr = meta
+        act, training, eps, momentum, deepchem, Cr, grad = meta
         if deepchem:
             (w_rel1, b_rel1, w_root1, w_rel2, b_rel2, w_root2, g1, be1, g2, be2, w_fc1, b_fc1, g3, be3) = params
         else:
@@ -132,7 +156,7 @@ class GraphNetFusedFn(torch.autograd.Function):
         g1, be1, g2, be2 = _pad(g1, (Ch,)), _pad(be1, (Ch,)), _pad(g2, (Ch,)), _pad(be2, (Ch,))
         if deepchem:
             w_fc1, b_fc1, g3, be3 = _pad(w_fc1, (C_FC, Ch)), L.f32c(b_fc1), L.f32c(g3), L.f32c(be3)
-        mean = 1 if graph.aggr == "mean" else 0
+        aggr = L.POOL[graph.aggr]
         f32 = dict(dtype=torch.float32, device=x.device)
         bf = dict(dtype=torch.bfloat16, device=x.device)
         nmax = call("pcc_gnn_max_blocks")
@@ -160,7 +184,7 @@ class GraphNetFusedFn(torch.autograd.Function):
         agg1 = torch.empty((M, F), **f32)
         z1 = torch.empty((M, Ch), **f32)
         nb = _nblk()
-        call("pcc_gnn_conv1_fwd", ptr(x), F, ptr(graph.rowptr_d), ptr(graph.col_d), ptr(graph.w_d), mean, ptr(w_rel1), ptr(w_root1),
+        call("pcc_gnn_conv1_fwd", ptr(x), F, ptr(graph.rowptr_d), ptr(graph.col_d), ptr(graph.w_d), aggr, ptr(w_rel1), ptr(w_root1),
              ptr(b_rel1), M, A, ptr(agg1), ptr(z1), ptr(part), C.byref(nb), dev, st)
         s1, t1, mu1, r1 = bn(0, Ch, g1, be1, nb.value, M)
         h1 = torch.empty((M, Ch), **bf)
@@ -169,8 +193,13 @@ class GraphNetFusedFn(torch.autograd.Function):
         agg2 = torch.empty((M, Ch), **bf)
         z2 = torch.empty((M, Ch), **f32)
         psum2 = None if deepchem else torch.empty((B, Ch), **f32)
-        call("pcc_gnn_conv_fwd", ptr(h1), ptr(graph.rowptr_d), ptr(graph.col_d), ptr(graph.w_d), mean, ptr(packed), ptr(b_rel2), M, A,
-             ptr(agg2), ptr(z2), ptr(part), ptr(membership) if not deepchem else None, ptr(psum2), B, C.byref(nb), dev, st)
+        # max aggregation: winner masks (16 bytes per edge) only when this step will run a backward
+        win = None
+        if graph.aggr == "max" and training and grad and any(ctx.needs_input_grad):
+            win = torch.empty((max(graph.E, 1), 16), dtype=torch.uint8, device=x.device)
+        call("pcc_gnn_conv_fwd", ptr(h1), ptr(graph.rowptr_d), ptr(graph.col_d), ptr(graph.w_d), aggr, ptr(packed), ptr(b_rel2), M, A,
+             ptr(agg2), ptr(z2), ptr(part), ptr(membership) if not deepchem else None, ptr(psum2), B, ptr(win), C.byref(nb), dev, st)
+        ctx.win = win
         s2, t2, mu2, r2 = bn(1, Ch, g2, be2, nb.value, M)
         counts = L.i64c(counts)
         ctx.graph, ctx.meta, ctx.shapes = graph, meta, (M, F, B)
@@ -195,7 +224,7 @@ class GraphNetFusedFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, G):
-        act, training, eps, momentum, deepchem, Cr = ctx.meta
+        act, training, eps, momentum, deepchem, Cr, _ = ctx.meta
         if not training:
             raise RuntimeError("the fused GraphNet backward uses batch statistics: call it in train() mode")
         graph = ctx.graph
@@ -254,9 +283,9 @@ class GraphNetFusedFn(torch.autograd.Function):
         call("pcc_gnn_reduce", ptr(cb_part), nb.value, Ch, ptr(d_b2), dev, st)
         d_wrel2, d_wroot2 = d_w2[:Cr, :Cr].contiguous(), d_w2[:Cr, Ch:Ch + Cr].contiguous()
         # ---- dh1 = droot + A^T dagg2 (+ bn1 sums)
-        rowptr_s, col_s, w_s = graph.by_src()
-        call("pcc_gnn_agg_bwd", ptr(dagg2), ptr(rowptr_s), ptr(col_s), ptr(w_s), ptr(droot), ptr(z1), ptr(mu1), ptr(r1), M, A,
-             ptr(stat), C.byref(nb), dev, st)
+        rowptr_s, col_s, w_s, pos_s = graph.by_src()
+        call("pcc_gnn_agg_bwd", ptr(dagg2), ptr(rowptr_s), ptr(col_s), ptr(w_s), L.POOL[graph.aggr], ptr(pos_s), ptr(ctx.win), ptr(droot),
+             ptr(z1), ptr(mu1), ptr(r1), M, A, ptr(stat), C.byref(nb), dev, st)
         c1b, c2b, d_g1, d_be1 = (torch.empty(Ch, **f32) for _ in range(4))
         call("pcc_gnn_bn_bwd_finalize", ptr(stat), nb.value, Ch, M, ptr(c1b), ptr(c2b), ptr(d_g1), ptr(d_be1), dev, st)
         # ---- conv1 backward (weights only: x needs no gradient)

@@ -178,7 +178,8 @@ def _fused_methods():
         bns = (self.bn1, self.bn2, self.bn3)
         bufs = [(b.running_mean, b.running_var) for b in bns]
         hidden = self.conv2.out_channels
-        meta = (self._act_name, self.training, float(self.bn1.eps), float(self.bn1.momentum), bool(self.deepchem_style), hidden)
+        meta = (self._act_name, self.training, float(self.bn1.eps), float(self.bn1.momentum), bool(self.deepchem_style), hidden,
+                torch.is_grad_enabled())
         params = (self.conv1.lin_rel.weight, self.conv1.lin_rel.bias, self.conv1.lin_root.weight,
                   self.conv2.lin_rel.weight, self.conv2.lin_rel.bias, self.conv2.lin_root.weight,
                   self.bn1.weight, self.bn1.bias, self.bn2.weight, self.bn2.bias)

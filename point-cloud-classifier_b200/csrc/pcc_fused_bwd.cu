@@ -76,8 +76,10 @@ __host__ __device__ inline BwdSmem bwd_smem(int H, int L) {
 //                                                                  the MMA accumulates onto accB), z_0 -> accA
 //                E: dZ_0 = dH_0 * act'(z_0) -> bufG (staged)
 // so the dgrad of the final layer runs under the h_0 epilogue and z of the last hidden layer is read
-// from TMEM once for both of its uses.
-template <int H, int ACT>
+// from TMEM once for both of its uses.  Max pooling with L = 3 (`pipe` below) hands the h_0 and dZ_1 images
+// over slab by slab and rotates the two accumulators, so that z_1, dH_0 and the next tile's z_0 run under the
+// epilogue passes; with ReLU, dZ_0 takes act'(z_0) from bits kept by the h_0 pass instead of a second z_0 GEMM.
+template <int H, int ACT, bool PIPE>
 __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const BwdSmem lay = bwd_smem(H, p.L);
@@ -92,7 +94,8 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
   uint64_t* accA_ready = bars + 2 * kRingB + 1;  // z in accA complete
   uint64_t* accB_ready = bars + 2 * kRingB + 2;  // dH in accB complete
   uint64_t* wf_ready = bars + 2 * kRingB + 3;    // virtual-row mode: rows of the final weight image landed in bufG
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kRingB + 4);
+  uint64_t* slab_ready = bars + 2 * kRingB + 4;  // [4] max pooling, L = 3: 64-column slab s of h_0 / dZ_1 written
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kRingB + 8);
 
   constexpr uint32_t SLAB = w_slab_bytes(H);
   constexpr uint32_t X_LBO = kTileM * 16;
@@ -113,6 +116,8 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
     mbar_init(accA_ready, 1);
     mbar_init(accB_ready, 1);
     mbar_init(wf_ready, 1);
+    if (PIPE)
+      for (int i = 0; i < 4; ++i) mbar_init(&slab_ready[i], kEpiWarps);
     fence_mbar_init();
   }
   if (warp == kMmaWarp) tmem_alloc<512>(tmem_slot);
@@ -136,13 +141,31 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
   // epilogue: that epilogue also stores act'(z_0) there (bf16), so the tile needs neither a second z_0 GEMM nor a second
   // activation evaluation for dZ_0; dZ_1 is written over h_0 (already staged) and feeds the dgrad from there.
   const bool bcast3 = bcast && p.L == 3;
+  // pipe (max pooling, two hidden layers): every GEMM runs under the epilogue pass that feeds it.  The two 256-column
+  // accumulators rotate: tile t holds z_0 and then dH_0 in X, z_1 in Y, and X / Y swap every tile, so
+  //   h_0 pass (reads X)        | z_1 = h_0 W_1^T -> Y, K slab s issued as soon as h_0 slab s is written
+  //   h_1 / dZ_1 pass (reads Y) | dH_0 = dZ_1 W_1 -> X, K slab s issued as soon as dZ_1 slab s is written
+  //   dZ_0 pass (reads X)       | z_0 of the next tile -> Y (ReLU; its x tile is staged before this pass)
+  // Within each GEMM the K order is that of a plain gemm(), so the accumulators hold the same bits.  A template
+  // parameter (the host sets it exactly when p.virt == 1 and p.L == 3), so the other modes compile without it.
+  constexpr bool pipe = PIPE;
+  // ReLU: act'(z_0 + b_0) is the predicate z_0 + b_0 > 0, which the h_0 pass keeps as a bit mask in registers (every
+  // thread owns the same row and column chunks in the h_0 and dZ_0 passes), so z_0 is not recomputed for dZ_0.  Other
+  // activations recompute z_0 into Y after the h_1 / dZ_1 pass.
+  constexpr bool mask0 = PIPE && ACT == PCC_ACT_RELU;
+  // wait trace of the producer and the MMA thread (tools/trace_bwd.py): pipelined variant only, so that the other modes
+  // compile without it
+  long long* const wtrace = PIPE ? p.trace : nullptr;
 
   if (warp == kProdWarp) {
     // ===================== producer: weight slabs in consumption order
     if (lane == 0) {
       uint32_t stage = 0, phase = 0;
+      int tn = 0;
       auto push = [&](const uint8_t* src, uint32_t bytes) {
+        trace_b(wtrace, 2, tn, 30);   // ring slot wait: begin / end
         mbar_wait(&empty[stage], phase ^ 1);
+        trace_b(wtrace, 2, tn, 31);
         mbar_arrive_expect_tx(&full[stage], bytes);
         bulk_g2s(ring + stage * SLAB, src, bytes, &full[stage]);
         if (++stage == kRingB) { stage = 0; phase ^= 1; }
@@ -154,7 +177,7 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
         if (L == 3) {
           push_layer(p.w_off[1]);                               // z_1
           push_layer(p.wt_off[1]);                              // dgrad of layer 1
-          if (!bcast3) push(p.wpack + p.w_off[0], (kK0 / 8) * W0_LBO);      // z_0 again
+          if (!bcast3 && !mask0) push(p.wpack + p.w_off[0], (kK0 / 8) * W0_LBO);      // z_0 again
         }
       }
     }
@@ -163,34 +186,85 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
     if (lane == 0) {
       constexpr uint32_t IDESC = make_idesc_bf16(128, H, 0, 0);
       uint32_t stage = 0, phase = 0, a_phase = 0;
+      int tn = 0;
       const uint32_t g_base = smem_u32(bufG), h_base = smem_u32(bufH), r_base = smem_u32(ring);
-      auto wait_a = [&]() { mbar_wait(a_ready, a_phase); a_phase ^= 1; tc_fence_after(); };
-      // D[acc] (+)= act[128 x H] (SW128 image) * streamed weight image^T
-      auto gemm = [&](uint32_t act_base, uint32_t acc_col, bool accumulate_first) {
-        for (int s = 0; s < NSLAB; ++s) {
-          mbar_wait(&full[stage], phase);
-          tc_fence_after();
-          const uint32_t w_slab = r_base + stage * SLAB;
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks)
-            umma_bf16(tmem + acc_col, make_smem_desc_sw128_k(act_base + s * kActSlab + ks * 32),
-                      make_smem_desc_sw128_k(w_slab + ks * 32), IDESC, ((s | ks) != 0) || accumulate_first);
-          umma_commit(&empty[stage]);
-          if (++stage == kRingB) { stage = 0; phase ^= 1; }
-        }
-      };
-      // z_0 = x tile (un-swizzled image at the head of bufH) * W_0^T -> accA
-      auto gemm0 = [&]() {
-        mbar_wait(&full[stage], phase);
+      // trace ids of the MMA thread: 40/41 operand hand-over wait begin/end, 42/43 weight slab wait begin/end
+      auto wait_a = [&]() {
+        trace_b(wtrace, 1, tn, 40);
+        mbar_wait(a_ready, a_phase);
+        trace_b(wtrace, 1, tn, 41);
+        a_phase ^= 1;
         tc_fence_after();
-        umma_bf16(tmem + ACC_A, make_smem_desc(h_base, X_LBO, 128), make_smem_desc(r_base + stage * SLAB, W0_LBO, 128),
+      };
+      auto wait_full = [&]() {
+        trace_b(wtrace, 1, tn, 42);
+        mbar_wait(&full[stage], phase);
+        trace_b(wtrace, 1, tn, 43);
+        tc_fence_after();
+      };
+      // D[acc] (+)= act[:, K slab s] (SW128 image) * streamed weight slab^T
+      auto gemm_slab = [&](uint32_t act_base, uint32_t acc_col, int s, bool accumulate_first) {
+        wait_full();
+        const uint32_t w_slab = r_base + stage * SLAB;
+#pragma unroll
+        for (int ks = 0; ks < 4; ++ks)
+          umma_bf16(tmem + acc_col, make_smem_desc_sw128_k(act_base + s * kActSlab + ks * 32),
+                    make_smem_desc_sw128_k(w_slab + ks * 32), IDESC, ((s | ks) != 0) || accumulate_first);
+        umma_commit(&empty[stage]);
+        if (++stage == kRingB) { stage = 0; phase ^= 1; }
+      };
+      // D[acc] (+)= act[128 x H] * streamed weight image^T
+      auto gemm = [&](uint32_t act_base, uint32_t acc_col, bool accumulate_first) {
+        for (int s = 0; s < NSLAB; ++s) gemm_slab(act_base, acc_col, s, accumulate_first);
+      };
+      // z_0 = x tile (un-swizzled image at the head of bufH) * W_0^T -> acc
+      auto gemm0 = [&](uint32_t acc_col) {
+        wait_full();
+        umma_bf16(tmem + acc_col, make_smem_desc(h_base, X_LBO, 128), make_smem_desc(r_base + stage * SLAB, W0_LBO, 128),
                   IDESC, 0);
         umma_commit(&empty[stage]);
         if (++stage == kRingB) { stage = 0; phase ^= 1; }
       };
+      if (pipe) {
+        const bool res = (p.res_mask >> 1) & 1;
+        uint32_t sl_phase = 0, accX = ACC_A;
+        auto wait_slab = [&](int s) {  // trace ids 44/45: slab hand-over wait begin/end
+          trace_b(wtrace, 1, tn, 44);
+          mbar_wait(&slab_ready[s], sl_phase);
+          trace_b(wtrace, 1, tn, 45);
+          tc_fence_after();
+        };
+        for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+          const uint32_t accY = ACC_A + ACC_B - accX;
+          wait_a();                                 // x tile staged (ReLU: during the previous tile's h_1 / dZ_1 pass)
+          gemm0(accX);
+          umma_commit(accA_ready);
+          for (int s = 0; s < NSLAB; ++s) {         // z_1 under the h_0 pass; X is free once its last slab is handed over
+            wait_slab(s);
+            gemm_slab(h_base, accY, s, false);
+          }
+          sl_phase ^= 1;
+          umma_commit(accA_ready);
+          // ResidualBlock: dH_1 is stored into X during the dZ_1 pass and the dgrad accumulates onto all of it
+          if (res)
+            for (int s = 0; s < NSLAB; ++s) wait_slab(s);
+          for (int s = 0; s < NSLAB; ++s) {         // dH_0 (+ dH_1) under the h_1 / dZ_1 pass
+            wait_slab(s);
+            gemm_slab(g_base, accX, s, res);
+          }
+          sl_phase ^= 1;
+          umma_commit(accB_ready);
+          if (!mask0) {
+            wait_a();                               // x tile staged again
+            gemm0(accY);                            // z_0 again, into Y (read by the h_1 / dZ_1 pass before)
+            umma_commit(accA_ready);
+          }
+          accX = accY;
+        }
+      } else
       for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
         wait_a();                                   // x tile staged
-        gemm0();
+        gemm0(ACC_A);
         umma_commit(accA_ready);
         if (!virt) {
           wait_a();                                 // dZ of the final layer built
@@ -206,7 +280,7 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
           umma_commit(accB_ready);
           if (!bcast3) {
             wait_a();                               // x tile staged again
-            gemm0();                                // z_0 again
+            gemm0(ACC_A);                           // z_0 again
             umma_commit(accA_ready);
           }
         }
@@ -226,13 +300,32 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
       for (int j = 0; j < kK0; ++j)
         xnext[j] = (grp == 0 && j < d && row < p.n && tile < p.num_tiles) ? __ldg(p.x + row * d + j) : 0.f;
     };
-    auto stage_x = [&]() {  // x tile -> un-swizzled [2][128][8] image at the head of bufH
+    auto stage_x = [&](const float (&xv)[kK0]) {  // x tile -> un-swizzled [2][128][8] image at the head of bufH
       if (grp == 0) {
-        *reinterpret_cast<uint4*>(bufH + r * 16) = make_uint4(pack_bf16x2(xcur[0], xcur[1]), pack_bf16x2(xcur[2], xcur[3]),
-                                                              pack_bf16x2(xcur[4], xcur[5]), pack_bf16x2(xcur[6], xcur[7]));
+        *reinterpret_cast<uint4*>(bufH + r * 16) = make_uint4(pack_bf16x2(xv[0], xv[1]), pack_bf16x2(xv[2], xv[3]),
+                                                              pack_bf16x2(xv[4], xv[5]), pack_bf16x2(xv[6], xv[7]));
         *reinterpret_cast<uint4*>(bufH + X_LBO + r * 16) =
-            make_uint4(pack_bf16x2(xcur[8], xcur[9]), pack_bf16x2(xcur[10], xcur[11]), pack_bf16x2(xcur[12], xcur[13]),
-                       pack_bf16x2(xcur[14], xcur[15]));
+            make_uint4(pack_bf16x2(xv[8], xv[9]), pack_bf16x2(xv[10], xv[11]), pack_bf16x2(xv[12], xv[13]),
+                       pack_bf16x2(xv[14], xv[15]));
+      }
+    };
+    // mask0: the next x tile as bf16 pairs (the packing of stage_x).  It is loaded just before the z_1 wait and staged
+    // after the h_1 / dZ_1 pass; the loads issue together and only 8 registers stay live (a float prefetch at the
+    // start of the tile was spilled load by load, each spill store waiting for its load)
+    uint32_t xpk[kK0 / 2];
+    auto load_xpk = [&](int64_t tile) {
+      const int64_t row = tile * kTileM + r;
+      float v[kK0];
+#pragma unroll
+      for (int j = 0; j < kK0; ++j)
+        v[j] = (grp == 0 && j < d && row < p.n && tile < p.num_tiles) ? __ldg(p.x + row * d + j) : 0.f;
+#pragma unroll
+      for (int k = 0; k < kK0 / 2; ++k) xpk[k] = pack_bf16x2(v[2 * k], v[2 * k + 1]);
+    };
+    auto stage_xpk = [&]() {
+      if (grp == 0) {
+        *reinterpret_cast<uint4*>(bufH + r * 16) = make_uint4(xpk[0], xpk[1], xpk[2], xpk[3]);
+        *reinterpret_cast<uint4*>(bufH + X_LBO + r * 16) = make_uint4(xpk[4], xpk[5], xpk[6], xpk[7]);
       }
     };
     // buffer hand-over with the bulk stores issued by thread 0
@@ -259,20 +352,37 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
     auto wait_A = [&]() { mbar_wait(accA_ready, phA); phA ^= 1; tc_fence_after(); };
     auto wait_B = [&]() { mbar_wait(accB_ready, phB); phB ^= 1; tc_fence_after(); };
     auto arrive_a = [&]() { tc_fence_before(); fence_proxy_async(); mbar_arrive_warp(a_ready); };
-    // h = [old +] act(z + b) for one 8-column group (packed-pair math: two columns per instruction)
-    auto h_chunk8 = [&](const uint32_t* z, const float* bl, uint8_t* dst, bool res) {
+    auto arrive_slab = [&](int s) { tc_fence_before(); fence_proxy_async(); mbar_arrive_warp(&slab_ready[s]); };
+    // h = [old +] act(z + b) for one 8-column group (packed-pair math: two columns per instruction); returns the
+    // predicates z + b > 0 (ReLU: act'(z + b)) as bits 0..7
+    auto h_chunk8 = [&](const uint32_t* z, const float* bl, uint8_t* dst, bool res) -> uint32_t {
       const float4 b0 = *reinterpret_cast<const float4*>(bl);
       const float4 b1 = *reinterpret_cast<const float4*>(bl + 4);
       const uint64_t bb[4] = {f32x2(b0.x, b0.y), f32x2(b0.z, b0.w), f32x2(b1.x, b1.y), f32x2(b1.z, b1.w)};
       uint4 old = make_uint4(0u, 0u, 0u, 0u);
       if (res) old = *reinterpret_cast<const uint4*>(dst);
       const uint32_t oo[4] = {old.x, old.y, old.z, old.w};
+      uint32_t pk[4], m = 0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const uint64_t zb = fadd2(f32x2(__uint_as_float(z[2 * j]), __uint_as_float(z[2 * j + 1])), bb[j]);
+        float lo, hi;
+        f32x2_unpack(zb, lo, hi);
+        m |= (lo > 0.f ? 1u : 0u) << (2 * j) | (hi > 0.f ? 1u : 0u) << (2 * j + 1);
+        uint64_t o = act2<ACT>(zb);
+        if (res) o = fadd2(o, bf16x2_to_f32x2(oo[j]));
+        pk[j] = pack_bf16x2_pair(o);
+      }
+      *reinterpret_cast<uint4*>(dst) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+      return m;
+    };
+    // ReLU: dZ = dH * act'(z + b) for one 8-column group, act' given as the bits 0..7 of m: the same product as dz_chunk8
+    auto dzm_chunk8 = [&](const uint32_t* g, uint32_t m, uint8_t* dst) {
       uint32_t pk[4];
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        uint64_t o = act2<ACT>(fadd2(f32x2(__uint_as_float(z[2 * j]), __uint_as_float(z[2 * j + 1])), bb[j]));
-        if (res) o = fadd2(o, bf16x2_to_f32x2(oo[j]));
-        pk[j] = pack_bf16x2_pair(o);
+        const uint64_t da = f32x2((m >> (2 * j)) & 1u ? 1.f : 0.f, (m >> (2 * j + 1)) & 1u ? 1.f : 0.f);
+        pk[j] = pack_bf16x2_pair(fmul2(f32x2(__uint_as_float(g[2 * j]), __uint_as_float(g[2 * j + 1])), da));
       }
       *reinterpret_cast<uint4*>(dst) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
     };
@@ -327,37 +437,51 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
       *reinterpret_cast<uint4*>(gdst) = make_uint4(pg[0], pg[1], pg[2], pg[3]);
     };
 
-    load_x(blockIdx.x);
+    if (mask0) load_xpk(blockIdx.x);
+    else load_x(blockIdx.x);
     int tn = 0;
     const bool tr0 = threadIdx.x == 0;
 #define TRE(id) do { if (tr0) trace_b(p.trace, 0, tn, id); } while (0)
+    uint32_t accX = ACC_A;  // pipe: the accumulator of z_0 and dH_0 in this tile (the other one, Y, holds z_1)
     for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
       const int64_t r0 = tile * kTileM;
       const int64_t row = r0 + r;
+      const uint32_t accY = ACC_A + ACC_B - accX;
+      // layer-0 act' bits of this thread's chunks grp, grp + 2, ... in order (mask0; bit j of an entry = column j)
+      uint32_t mk[NCHUNK / 2];
+      if (!mask0) {
 #pragma unroll
-      for (int j = 0; j < kK0; ++j) xcur[j] = xnext[j];
+        for (int j = 0; j < kK0; ++j) xcur[j] = xnext[j];
+      }
       TRE(0);
-      stage_x();  // bufH is free: its last staging store (h_lh) was waited for before dZ_0 / at the previous tile
-      arrive_a();
+      if (!mask0 || tile == blockIdx.x) {
+        // bufH is free: its last staging store (h_lh) was waited for before dZ_0 / at the previous tile
+        if (mask0) stage_xpk();
+        else stage_x(xcur);
+        arrive_a();     // (mask0: staged after the previous tile's h_1 / dZ_1 pass)
+      }
       TRE(2);
-      load_x(tile + gridDim.x);
+      if (!mask0) load_x(tile + gridDim.x);
       // set of this thread's row (for the pooled-gradient scatter), precomputed; virtual-row mode: the row's
       // pooled gradient itself
       const int64_t myset = (!vmax && row < p.n) ? (int64_t)__ldg(p.row_set + row) : -1;
       const float scale = (!vmax && row < p.n) ? __ldg(p.row_scale + row) : 0.f;
-      const float gs = vmax ? ((row < p.n) ? __ldg(p.dpooled + row) : 0.f) : 1.f;
+      float gs = (vmax && !mask0) ? ((row < p.n) ? __ldg(p.dpooled + row) : 0.f) : 1.f;  // mask0: under the z_1 wait
+
+      // rows f0 .. f0+127 of the final weight image -> bufG (same SW128 layout as an activation image); thread 0, once
+      // the previous tile's dZ_0 store has finished reading bufG
+      auto load_wrows = [&]() {
+        const uint32_t f0 = (uint32_t)(r0 % H);
+        mbar_arrive_expect_tx(wf_ready, NSLAB * kActSlab);
+        for (int s = 0; s < NSLAB; ++s)
+          bulk_g2s(bufG + s * kActSlab, p.wpack + p.w_off[L - 1] + (size_t)s * SLAB + (size_t)f0 * 128, kActSlab, wf_ready);
+      };
 
       // ---- dZ of the final Linear from the pooled gradient (autograd of deep_sets.py:96-106)
-      acquire();  // the previous tile's dZ_0 store has finished reading bufG
+      if (!pipe) acquire();  // the previous tile's dZ_0 store has finished reading bufG (pipe: during the h_0 pass)
       TRE(1);
       if (vmax) {
-        // rows f0 .. f0+127 of the final weight image -> bufG (same SW128 layout as an activation image)
-        if (threadIdx.x == 0) {
-          const uint32_t f0 = (uint32_t)(r0 % H);
-          mbar_arrive_expect_tx(wf_ready, NSLAB * kActSlab);
-          for (int s = 0; s < NSLAB; ++s)
-            bulk_g2s(bufG + s * kActSlab, p.wpack + p.w_off[L - 1] + (size_t)s * SLAB + (size_t)f0 * 128, kActSlab, wf_ready);
-        }
+        if (!pipe && threadIdx.x == 0) load_wrows();
       } else if (!bcast3) {
         // the pooled-gradient rows of the sets that intersect this tile are staged one set at a time in a
         // scratch area of bufH (free until the h_0 epilogue) and broadcast from shared memory; a thread
@@ -434,25 +558,46 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
         TRE(5);
         const float* bl = biasS;
         uint32_t va[32], vb[32];
-        tmem_ld32(lane_base + ACC_A + grp * 32, va);
+        // one chunk of h_0; mask0 keeps its act' bits
+        auto h_chunk32 = [&](const uint32_t (&z)[32], int c) {
+          uint32_t m = 0;
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            m |= h_chunk8(z + q * 8, bl + c * 32 + q * 8, bufH + act_chunk_off(r, c * 32 + q * 8), false) << (8 * q);
+          if (mask0) {
+#pragma unroll
+            for (int k = 0; k + 1 < NCHUNK / 2; ++k) mk[k] = mk[k + 1];
+            mk[NCHUNK / 2 - 1] = m;
+          }
+        };
+        tmem_ld32(lane_base + accX + grp * 32, va);
 #pragma unroll 1
         for (int c = grp; c < NCHUNK; c += 4) {
           tmem_wait_ld();
-          if (c + 2 < NCHUNK) tmem_ld32(lane_base + ACC_A + (c + 2) * 32, vb);
-#pragma unroll
-          for (int q = 0; q < 4; ++q) h_chunk8(va + q * 8, bl + c * 32 + q * 8, bufH + act_chunk_off(r, c * 32 + q * 8), false);
+          if (c + 2 < NCHUNK) tmem_ld32(lane_base + accX + (c + 2) * 32, vb);
+          h_chunk32(va, c);
+          if (pipe) arrive_slab(c >> 1);  // the z_1 MMAs of this K slab can start
           if (c + 2 < NCHUNK) {
             tmem_wait_ld();
-            if (c + 4 < NCHUNK) tmem_ld32(lane_base + ACC_A + (c + 4) * 32, va);
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-              h_chunk8(vb + q * 8, bl + (c + 2) * 32 + q * 8, bufH + act_chunk_off(r, (c + 2) * 32 + q * 8), false);
+            if (c + 4 < NCHUNK) tmem_ld32(lane_base + accX + (c + 4) * 32, va);
+            h_chunk32(vb, c + 2);
+            if (pipe) arrive_slab((c + 2) >> 1);
           }
           // the two groups together have finished slabs (c - grp) / 2 and + 1
           store_slabs(p.stage_h[0] + (size_t)tile * BLOB, bufH, (c - grp) >> 1, (c + 2 < NCHUNK) ? 2 : 1, nullptr, nullptr);
+          // pipe: the dZ_0 store of the previous tile has long drained, so the weight rows that the h_1 / dZ_1 pass
+          // reads are fetched here instead of holding up the start of the tile (all but the h_0 store just issued)
+          if (pipe && c == grp && threadIdx.x == 0) {
+            bulk_wait_read1();
+            load_wrows();
+          }
         }
         TRE(6);
-        arrive_a();
+        if (!pipe) arrive_a();
+        if (mask0) {  // needed after the z_1 wait at the earliest
+          load_xpk(tile + gridDim.x);
+          gs = (row < p.n) ? __ldg(p.dpooled + row) : 0.f;
+        }
         TRE(7);
       }
 
@@ -502,10 +647,11 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
         }
         const bool res = (p.res_mask >> lh) & 1;
         const float* bl = biasS + lh * H;
+        const uint32_t zacc = pipe ? accY : ACC_A, gacc = pipe ? accX : ACC_B;
 #pragma unroll 1
         for (int c = grp; c < NCHUNK; c += 2) {
           uint32_t z[32], g[32];
-          tmem_ld32(lane_base + ACC_A + c * 32, z);
+          tmem_ld32(lane_base + zacc + c * 32, z);
           // dH_lh chunk: mode 1: W_{L-1}[f, 32 columns] * dpooled[row]; mode 2: the image built from G (overwritten below)
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
@@ -516,13 +662,17 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
             g[q * 8 + 6] = __float_as_uint(gs * bf16_lo(wv.w)); g[q * 8 + 7] = __float_as_uint(gs * bf16_hi(wv.w));
           }
           // ResidualBlock: dH_{lh-1} = dZ_lh W_lh + dH_lh — the dgrad MMA accumulates onto accB, so dH_lh goes there
-          if (res) tmem_st32(lane_base + ACC_B + c * 32, g);
+          if (res) tmem_st32(lane_base + gacc + c * 32, g);
           tmem_wait_ld();
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
             const uint32_t off = act_chunk_off(r, c * 32 + q * 8);
             if (bcast) dz_chunk8(z + q * 8, g + q * 8, bl + c * 32 + q * 8, bufG + off);
             else hdz_chunk8(z + q * 8, g + q * 8, bl + c * 32 + q * 8, bufH + off, bufG + off, res);
+          }
+          if (pipe) {  // the dgrad MMAs of this K slab can start (ResidualBlock: once dH_1 is in X, see the MMA thread)
+            if (res) tmem_wait_st();
+            arrive_slab(c >> 1);
           }
           if (bcast) store_slabs(p.stage_g[lh] + (size_t)tile * BLOB, bufG, c >> 1, 1, nullptr, nullptr);
           else store_slabs(p.stage_h[lh] + (size_t)tile * BLOB, bufH, c >> 1, 1, p.stage_g[lh] + (size_t)tile * BLOB, bufG);
@@ -549,9 +699,13 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
       TRE(12);
 
       if (L == 3) {
-        arrive_a();  // dZ_1 image complete: the dgrad of layer 1 can start while the staging stores drain
-        // h_1 staged out of bufH: its head can take the x tile again
-        if (threadIdx.x == 0) bulk_wait_read0();  // slab-wise stores: only the last slab pair can still be in flight
+        if (!pipe) arrive_a();  // dZ_1 image complete: the dgrad of layer 1 can start while the staging stores drain
+        // h_1 staged out of bufH: its head can take the x tile again.  Slab-wise stores: only the last slab pair can
+        // still be in flight; mask0 lets it drain under the dgrad (the x image lies in slab 0, bufG is acquired below)
+        if (threadIdx.x == 0) {
+          if (mask0) bulk_wait_read1();
+          else bulk_wait_read0();
+        }
         asm volatile("bar.sync 1, 256;" ::: "memory");
         TRE(13);
         if (bcast3) {
@@ -578,31 +732,56 @@ __global__ void __launch_bounds__(kThreads, 1) phi_bwd_chain_kernel(const BwdPar
             }
             store_slabs(p.stage_g[0] + (size_t)tile * BLOB, bufG, c >> 1, 1, nullptr, nullptr);
           }
-        } else {
-        stage_x();
-        arrive_a();
-        // ---- dZ_0 = dH_0 * act'(z_0 + b_0) -> bufG, staged
-        wait_B();
-        wait_A();
-        TRE(14);
-        acquire();
-        TRE(15);
-        const float* bl = biasS;
+        } else if (mask0) {
+          // the next tile's x -> bufH head: its z_0 GEMM (into Y) runs under this pass
+          if (tile + gridDim.x < p.num_tiles) {
+            stage_xpk();
+            arrive_a();
+          }
+          // ---- dZ_0 = dH_0 * act'(z_0 + b_0) with act' from the h_0 pass's bits -> bufG (the dgrad has read it), staged
+          wait_B();
+          TRE(14);
+          acquire();  // the last dZ_1 store has finished reading bufG
+          TRE(15);
 #pragma unroll 1
-        for (int c = grp; c < NCHUNK; c += 2) {
-          uint32_t z[32], g[32];
-          tmem_ld32(lane_base + ACC_A + c * 32, z);
-          tmem_ld32(lane_base + ACC_B + c * 32, g);
-          tmem_wait_ld();
+          for (int c = grp; c < NCHUNK; c += 2) {
+            uint32_t g[32];
+            tmem_ld32(lane_base + accX + c * 32, g);
+            const uint32_t m = mk[0];
 #pragma unroll
-          for (int q = 0; q < 4; ++q)
-            dz_chunk8(z + q * 8, g + q * 8, bl + c * 32 + q * 8, bufG + act_chunk_off(r, c * 32 + q * 8));
-          store_slabs(p.stage_g[0] + (size_t)tile * BLOB, bufG, c >> 1, 1, nullptr, nullptr);
-        }
+            for (int k = 0; k + 1 < NCHUNK / 2; ++k) mk[k] = mk[k + 1];
+            tmem_wait_ld();
+#pragma unroll
+            for (int q = 0; q < 4; ++q) dzm_chunk8(g + q * 8, m >> (8 * q), bufG + act_chunk_off(r, c * 32 + q * 8));
+            store_slabs(p.stage_g[0] + (size_t)tile * BLOB, bufG, c >> 1, 1, nullptr, nullptr);
+          }
+        } else {
+          stage_x(xcur);
+          arrive_a();
+          // ---- dZ_0 = dH_0 * act'(z_0 + b_0) -> bufG, staged (pipe: z_0 recomputed into Y, dH_0 in X)
+          wait_B();
+          wait_A();
+          TRE(14);
+          acquire();
+          TRE(15);
+          const float* bl = biasS;
+          const uint32_t zacc = pipe ? accY : ACC_A, gacc = pipe ? accX : ACC_B;
+#pragma unroll 1
+          for (int c = grp; c < NCHUNK; c += 2) {
+            uint32_t z[32], g[32];
+            tmem_ld32(lane_base + zacc + c * 32, z);
+            tmem_ld32(lane_base + gacc + c * 32, g);
+            tmem_wait_ld();
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+              dz_chunk8(z + q * 8, g + q * 8, bl + c * 32 + q * 8, bufG + act_chunk_off(r, c * 32 + q * 8));
+            store_slabs(p.stage_g[0] + (size_t)tile * BLOB, bufG, c >> 1, 1, nullptr, nullptr);
+          }
         }
         TRE(16);
         TRE(17);
       }
+      if (pipe) accX = accY;
     }
 #undef TRE
     if (threadIdx.x == 0) bulk_wait0();
@@ -1020,7 +1199,7 @@ __global__ void set_bscale_kernel(const int64_t* __restrict__ offsets, int64_t B
 template <int H, int ACT>
 static int launch_chain(const BwdParams& p, int grid, cudaStream_t st) {
   const BwdSmem lay = bwd_smem(H, p.L);
-  auto kern = phi_bwd_chain_kernel<H, ACT>;
+  auto kern = (p.virt == 1 && p.L == 3) ? phi_bwd_chain_kernel<H, ACT, true> : phi_bwd_chain_kernel<H, ACT, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total);
   if (e != cudaSuccess) return fail("pcc_deepsets_phi_pool_bwd", cudaGetErrorString(e));
   {

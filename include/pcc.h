@@ -380,6 +380,9 @@ int pcc_debug_set_trace(void* device_buf);
 /* forward kernel selection for H = 256 without commuted pooling: 1 = CTA-pair kernel (cta_group::2, default; env
  * PCC_FWD_PAIR=0 disables), 0 = one CTA per SM.  Both compute the same function; tests compare them. */
 int pcc_debug_set_fwd_pair(int on);
+/* backward chain schedule for max pooling with two hidden layers: 1 = pipelined (the GEMMs run under the epilogue
+ * passes, default), 0 = serial (one GEMM after another).  Both compute the same function; tests compare them. */
+int pcc_debug_set_bwd_pipe(int on);
 /* programmatic dependent launch between the kernels of the DeepSets train step (griddepcontrol: a kernel is
  * scheduled while its predecessor drains and waits for it before its first global access): 1 = on (default; env
  * PCC_PDL=0 disables), 0 = plain stream-ordered launches.  Same results either way; tests compare them. */

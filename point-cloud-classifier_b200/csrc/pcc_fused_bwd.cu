@@ -1196,10 +1196,13 @@ __global__ void set_bscale_kernel(const int64_t* __restrict__ offsets, int64_t B
   bscale[b] = (n <= 0.f) ? 0.f : (pooling == PCC_POOL_SUM ? sqrtf(n) : 1.f);
 }
 
+static int g_bwd_pipe = 1;  // pcc_debug_set_bwd_pipe: 0 runs max pooling with two hidden layers on the serial schedule
+
 template <int H, int ACT>
 static int launch_chain(const BwdParams& p, int grid, cudaStream_t st) {
   const BwdSmem lay = bwd_smem(H, p.L);
-  auto kern = (p.virt == 1 && p.L == 3) ? phi_bwd_chain_kernel<H, ACT, true> : phi_bwd_chain_kernel<H, ACT, false>;
+  auto kern = (p.virt == 1 && p.L == 3 && g_bwd_pipe) ? phi_bwd_chain_kernel<H, ACT, true>
+                                                       : phi_bwd_chain_kernel<H, ACT, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total);
   if (e != cudaSuccess) return fail("pcc_deepsets_phi_pool_bwd", cudaGetErrorString(e));
   {
@@ -1224,6 +1227,11 @@ static int launch_wgrad(const BwdParams& p, int grid, cudaStream_t st) {
 }  // namespace pcc
 
 using namespace pcc;
+
+extern "C" int pcc_debug_set_bwd_pipe(int on) {
+  pcc::g_bwd_pipe = on ? 1 : 0;
+  return 0;
+}
 
 extern "C" int pcc_deepsets_phi_pool_bwd(const pcc_phi_desc* d, const float* x, const int64_t* offsets, int64_t n,
                                          int64_t B, const float* dpooled, const int32_t* argmax, float* const* dw,

@@ -96,6 +96,7 @@ _SIGS = {
     "pcc_prof_read": [_i32, C.POINTER(C.c_double), C.POINTER(C.c_int64)],
     "pcc_debug_set_trace": [_vp],
     "pcc_debug_set_fwd_pair": [_i32],
+    "pcc_debug_set_bwd_pipe": [_i32],
     "pcc_debug_set_pdl": [_i32],
     "pcc_selftest_umma": [_i32, _vp, _i32, _vp],
     "pcc_selftest_fp32_peak": [_vp, _i32, _i32, _i32, _vp],

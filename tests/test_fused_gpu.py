@@ -101,6 +101,14 @@ CASES = [
     ("gelu", "max", True, 256, 2, 3, [300, 129, 1, 700, 64]),
     ("silu", "max", False, 256, 1, 6, [128, 128, 128, 5, 250]),
     ("relu", "max", False, 256, 1, 3, [1000, 24]),
+    # max pooling, two hidden layers, B*H < sum N: the backward runs on the B*H argmax rows through the pipelined chain
+    # schedule; the first two have more of those 128-row tiles (160) than a B200 has SMs.  (ReLU + ResidualBlock is
+    # left to test_maxpool_bwd_chain_gpu.py: on a 6-set batch its bf16 residual sum moves pooled by ~1e-3, enough to
+    # flip a rho ReLU against the bf16-operand oracle and move every gradient by ~6e-2.)
+    ("silu", "max", True, 256, 2, 3, [200 + (37 * i) % 201 for i in range(80)]),
+    ("silu", "max", False, 128, 2, 1, [1 + (53 * i) % 300 for i in range(160)]),
+    ("gelu", "max", False, 256, 2, 5, [700, 3, 129, 1000, 64]),
+    ("relu", "max", False, 128, 2, 7, [300, 1, 129, 500, 64, 2]),
 ]
 
 
@@ -324,17 +332,27 @@ def test_dependent_launch_matches_stream_ordered_launch(pooling, act):
             assert torch.equal(ga, gb)
 
 
-@pytest.mark.parametrize("pool,H", [("sum", 128), ("mean", 256), ("max", 256)])
-def test_interior_empty_sets(pool, H):
+@pytest.mark.parametrize("pool,H,virtual", [pytest.param("sum", 128, False, id="sum-128"),
+                                            pytest.param("mean", 256, False, id="mean-256"),
+                                            pytest.param("max", 256, False, id="max-256"),
+                                            pytest.param("max", 256, True, id="max-256-virtual")])
+def test_interior_empty_sets(pool, H, virtual):
     """Sets without points inside the index range (a gap in idx, or an explicit num_sets): the library defines their
     pooled row as 0 and they receive no gradient.  One 128-row tile here intersects 328 sets (64 one-point sets,
     200 EMPTY ones, 64 one-point sets): the commuted sum / mean pooling runs its pooling MMA in chunks of <= 128 sets;
-    max pooling must not route the gradient of an empty set (argmax -1) to row 0."""
+    max pooling must not route the gradient of an empty set (argmax -1) to row 0.  `virtual`: more points than
+    num_sets * H, so the max-pool backward runs on the gathered argmax rows, where an empty set's rows are clamped to
+    row 0 and carry a zeroed pooled gradient (empty sets 1-3 and 5 inside, 8-11 trailing)."""
     d, act = 3, "gelu"
     cfg = _cfg(act, pool, False, H, 2, d)
     sd = O.init_state_dict(cfg, seed=91)
-    ids = list(range(64)) + list(range(264, 328)) + [328] * 300 + [330] * 5
-    num_sets = 480                                           # 149 trailing empty sets as well
+    if virtual:
+        ids = [0] * 1500 + [4] * 900 + [6] * 700 + [7] * 400
+        num_sets = 12
+        assert len(ids) > num_sets * H
+    else:
+        ids = list(range(64)) + list(range(264, 328)) + [328] * 300 + [330] * 5
+        num_sets = 480                                       # 149 trailing empty sets as well
     idx = torch.tensor(ids, dtype=torch.long)
     g = torch.Generator().manual_seed(92)
     x = torch.randn(len(ids), d, generator=g)
